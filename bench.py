@@ -11,6 +11,8 @@ Contract: python bench.py --gpus N --steps K --warmup W   (torchrun for N>1) pri
   cpu_baseline: the NumPy oracle (port of the reference; Theano is not installable) on the host cores, bounded sample
 --impl reference : times that CPU port alone (rank 0 only), same metric / config.
 --workload cfg1|cfg2|cfg2x|cfg3|cfg4 : the other BASELINE.json configurations (default cfg2 = the headline)
+--dump-outputs DIR : after the timed steps, DIR/<name>.npy holds what they computed (see dump_outputs); the inputs are seeded,
+            so two builds run with the same arguments can be compared output for output
 """
 import argparse
 import json
@@ -24,6 +26,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 # BASELINE.json configs; shapes from SURVEY.md section 8(d).  cfg2 = configs[1] is the headline (param_samples/rsc15_bpr-max.py).
 WORKLOADS = {
@@ -49,6 +52,24 @@ WORKLOADS = {
                  published_src='RetailRocket BPR-max shared, 1xGRU(224), B=80, A30 (README.md:153-169; nearest published shape)'),
 }
 SAMPLE_STORE = 10000000
+DUMP_ROWS = 16384                   # item-table rows kept by --dump-outputs: under 64 MB in all at every workload
+
+
+def dump_outputs(eng, names, costs, n_items, out_dir):
+    """What the timed steps computed, as float32 DIR/<name>.npy: `cost` (one per timed mini-batch, the last is the last step's)
+    and, as they stand after the last step, every parameter and the GRU hidden state H<i>.  Tables with one row per item and more
+    than DUMP_ROWS items are cut to a fixed seeded sample of rows, whose item ids `item_rows` holds."""
+    rows = np.sort(np.random.RandomState(0).choice(n_items, DUMP_ROWS, replace=False)) if n_items > DUMP_ROWS else None
+    out = {'cost': np.asarray(costs, dtype=np.float32)}
+    for name in names:
+        a = eng.get(name)
+        out[name] = a[rows] if rows is not None and a.shape[0] == n_items else a
+    if rows is not None:
+        out['item_rows'] = rows.astype(np.float32)
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20, 'dump larger than 64 MB'
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def algo_bytes_step(mk):
@@ -251,10 +272,15 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--replicated', action='store_true', help='N>1: replicated tables + NCCL exchange (round-1 path) instead of row sharding')
     ap.add_argument('--step-mode', type=int, default=2, help='0 per-phase kernels (CUDA graph), 1 persistent kernel, 2 role-specialised persistent kernel (default), 3 = 2 with the GRU phases on one thread-block cluster')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the costs of the timed steps and the parameters after the last one to DIR/<name>.npy (one GPU)')
     args = ap.parse_args()
     rank = int(os.environ.get('RANK', '0'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (world > 1 or args.impl != 'b200'):
+        ap.error('--dump-outputs needs the b200 path on one GPU')
     if args.impl == 'reference':
         run_reference(args, rank, world)
         return
@@ -357,6 +383,8 @@ def main():
         wall = time.time() - t0
         costs = np.concatenate(cost_parts)
         launches = eng.kernel_launches() - launches0
+        if args.dump_outputs:                    # before the e2e arm trains on
+            dump_outputs(eng, sorted(host) + ['H%d' % i for i in range(len(mk['layers']))], costs, wl['n_items'], args.dump_outputs)
         if dist is not None:
             t = torch.tensor([dev_ms], device='cuda'); dist.all_reduce(t, op=dist.ReduceOp.MAX); dev_ms = float(t.item())
         value = world * K / (dev_ms / 1000.0)

@@ -73,3 +73,89 @@ def fit_data(orc, g, tr):
 def epoch_order(g, d, e):
     """session order of epoch e: recorded np.random.permutation for train_random_order (gru4rec.py:593), else base_order"""
     return g['epoch_orders'][e] if 'epoch_orders' in g else d['base_order']
+
+
+# ---- datatools cases (tests/golden/datatools_cases.json, made by oracle/make_standalone_golden.py) ----
+def datatools_cases():
+    """(frame, sort columns, any_order_first_dim) of the 192 datatools comparisons, in a fixed seeded order: sorted, partly
+    sorted, grouped-but-unordered and random frames of 1 to 300 rows."""
+    rs = np.random.RandomState(0)
+    for n in (1, 2, 50, 300):
+        for trial in range(8):
+            df = pd.DataFrame({'SessionId': rs.randint(0, max(2, n // 4), n), 'Time': rs.randint(0, 40, n), 'ItemId': rs.randint(0, 9, n)})
+            if trial % 4 == 1: df = df.sort_values(['SessionId', 'Time']).reset_index(drop=True)
+            if trial % 4 == 2: df = df.sort_values(['SessionId', 'Time', 'ItemId']).reset_index(drop=True)
+            if trial % 4 == 3:      # sessions grouped but in arbitrary order
+                df = df.sort_values(['SessionId', 'Time']).reset_index(drop=True)
+                df = pd.concat([df[df.SessionId == s] for s in rs.permutation(df['SessionId'].unique())]).reset_index(drop=True)
+            for cols in (['SessionId', 'Time'], ['SessionId', 'Time', 'ItemId'], ['SessionId']):
+                for any_order in (False, True):
+                    yield df.copy(), cols, any_order
+
+
+def datatools_outcome(sort_if_needed, compute_offset, df, cols, any_order):
+    """What sort_if_needed (printed decision, frame left in place) and compute_offset do to one case: the printed lines without
+    the timing line, and SHA-256 digests of the frame (index, column names, dtypes, values) and of the offsets (dtype, values)."""
+    import contextlib, hashlib, io
+    buf = io.StringIO()
+    with contextlib.redirect_stdout(buf):
+        sort_if_needed(df, cols, any_order)
+    h = hashlib.sha256(np.asarray(df.index.values, dtype=np.int64).tobytes())
+    for c in df.columns:
+        h.update(('%s:%s' % (c, df[c].dtype)).encode()); h.update(np.ascontiguousarray(df[c].values).tobytes())
+    off = compute_offset(df, 'SessionId')
+    return {'stdout': [l for l in buf.getvalue().splitlines() if not l.startswith('Data is sorted in')], 'frame_sha256': h.hexdigest(),
+            'offset_sha256': hashlib.sha256(str(off.dtype).encode() + np.ascontiguousarray(off).tobytes()).hexdigest()}
+
+
+# ---- pickle compatibility (tests/golden/bprmax_none.b200model.pickle, made by oracle/make_standalone_golden.py) ----
+def b200_model_from_golden(g):
+    """This project's class holding the reference's final weights of golden run `g`, ready for savemodel()."""
+    import gru4rec
+    m = gru4rec.GRU4Rec(**g['model_kwargs'])
+    m.n_items = int(g['n_items'])
+    m.itemidmap = pd.Series(data=np.arange(m.n_items), index=g['itemidmap_index'], name='ItemIdx')
+    fw = init_weights(g, 'final_')
+    m._host = {'Wx0': fw['Wx'][0], 'Wh0': fw['Wh'][0], 'Wrz0': fw['Wrz'][0], 'Bh0': fw['Bh'][0], 'Wy': fw['Wy'], 'By': fw['By']}
+    m.error_during_train = False
+    return m
+
+
+def pickle_structure(path):
+    """The content of a model pickle as plain comparable values, without importing any class it names from `gru4rec`: objects
+    of those classes become (class name, state), bound methods taken from them become (class name, method name), arrays
+    become (dtype, shape, bytes), pandas objects (type, name, index, values)."""
+    import pickle
+
+    class Stand(object):
+        def __setstate__(self, st):
+            self.__dict__['_state'] = st
+
+        def __getattr__(self, name):
+            if name.startswith('__'):
+                raise AttributeError(name)
+            return ('bound method', type(self).__name__, name)
+
+    stand_ins = {}
+
+    class Unpickler(pickle.Unpickler):
+        def find_class(self, module, name):
+            if module == 'gru4rec':
+                return stand_ins.setdefault(name, type(name, (Stand,), {}))
+            return pickle.Unpickler.find_class(self, module, name)
+
+    def plain(v):
+        if isinstance(v, Stand):
+            return ('object', type(v).__name__, plain(v.__dict__.get('_state')))
+        if isinstance(v, dict):
+            return ('dict', sorted((k, plain(x)) for k, x in v.items()))
+        if isinstance(v, (list, tuple)):
+            return (type(v).__name__, [plain(x) for x in v])
+        if isinstance(v, np.ndarray):
+            return ('ndarray', v.dtype.str, v.shape, v.tobytes())
+        if isinstance(v, (pd.Series, pd.Index)):
+            return (type(v).__name__, v.name, plain(np.asarray(v.index if isinstance(v, pd.Series) else [])), plain(np.asarray(v.values)))
+        return (type(v).__name__, v)
+
+    with open(path, 'rb') as f:
+        return plain(Unpickler(f).load())

@@ -127,80 +127,33 @@ def test_loadmodel_reads_reference_written_pickle():
 
 
 def test_pickle_written_here_loads_into_the_reference_class(tmp_path):
-    """savemodel() of this class -> the REFERENCE's GRU4Rec.loadmodel + evaluate_gpu (run on the Theano shim) reproduce the
-    oracle's Recall/MRR.  Needs /root/reference (not present on the GPU box)."""
-    import subprocess, sys, json
-    if not os.path.exists('/root/reference/gru4rec.py'):
-        pytest.skip('reference tree not available')
-    import gru4rec
-    import pandas as pd
-    from golden_utils import load_golden, frames, init_weights
+    """savemodel() of this class writes what tests/golden/bprmax_none.b200model.pickle holds -- same classes, state keys, types
+    and values.  The REFERENCE's GRU4Rec.loadmodel + evaluate_gpu (run on the Theano shim by oracle/make_standalone_golden.py)
+    loaded that pickle and reproduced the oracle's Recall/MRR, recorded in bprmax_none.b200model.json."""
+    import json
+    from golden_utils import load_golden, b200_model_from_golden, pickle_structure, GOLDEN_DIR
     g = load_golden('bprmax_none')
-    mk = g['model_kwargs']
-    _, te = frames(g)
-    m = gru4rec.GRU4Rec(**mk)
-    m.n_items = int(g['n_items'])
-    m.itemidmap = pd.Series(data=np.arange(m.n_items), index=g['itemidmap_index'], name='ItemIdx')
-    fw = init_weights(g, 'final_')
-    m._host = {'Wx0': fw['Wx'][0], 'Wh0': fw['Wh'][0], 'Wrz0': fw['Wrz'][0], 'Bh0': fw['Bh'][0], 'Wy': fw['Wy'], 'By': fw['By']}
-    m.error_during_train = False
     fn = str(tmp_path / 'b200_model.pickle')
-    m.savemodel(fn)
-    te_fn = str(tmp_path / 'test.pickle'); te.to_pickle(te_fn)
-    code = (
-        "import sys, os, io, json, contextlib\n"
-        "sys.path.insert(0, %r); import theano_shim; theano_shim.install()\n"
-        "sys.path.insert(0, '/root/reference'); cwd = os.getcwd()\n"
-        "import gru4rec as ref, evaluation as ev, pandas as pd; os.chdir(cwd)\n"
-        "g = ref.GRU4Rec.loadmodel(%r)\n"
-        "assert type(g).__module__ == 'gru4rec' and hasattr(g.Wy, 'get_value')\n"
-        "te = pd.read_pickle(%r)\n"
-        "buf = io.StringIO()\n"
-        "with contextlib.redirect_stdout(buf): rec, mrr = ev.evaluate_gpu(g, te, cut_off=[1, 5, 20], batch_size=7)\n"
-        "print(json.dumps([[float(x) for x in rec], [float(x) for x in mrr]]))\n"
-    ) % (os.path.join(ROOT, 'oracle'), fn, te_fn)
-    out = subprocess.run([sys.executable, '-c', code], capture_output=True, text=True, timeout=300, cwd=str(tmp_path))
-    assert out.returncode == 0, out.stderr[-2000:]
-    rec, mrr = json.loads(out.stdout.strip().splitlines()[-1])
-    np.testing.assert_allclose(rec, g['eval_standard_recall'], rtol=1e-6)
-    np.testing.assert_allclose(mrr, g['eval_standard_mrr'], rtol=1e-6)
+    b200_model_from_golden(g).savemodel(fn)
+    assert pickle_structure(fn) == pickle_structure(os.path.join(GOLDEN_DIR, 'bprmax_none.b200model.pickle'))
+    ref = json.load(open(os.path.join(GOLDEN_DIR, 'bprmax_none.b200model.json')))
+    np.testing.assert_allclose(ref['recall'], g['eval_standard_recall'], rtol=1e-6)
+    np.testing.assert_allclose(ref['mrr'], g['eval_standard_mrr'], rtol=1e-6)
 
 
 def test_datatools_behaves_like_the_reference_module():
-    """gru4rec_b200/datatools.py is an independent implementation; wherever the reference checkout is available (this container,
-    not the GPU box) its datatools.py -- plain pandas/NumPy, importable without Theano -- is run side by side on random frames:
-    same printed decision, same in-place result, same int32 offsets."""
-    import io, contextlib, importlib.util
-    import pandas as pd
-    ref_path = '/root/reference/datatools.py'
-    if not os.path.exists(ref_path):
-        pytest.skip('reference checkout not available')
-    spec = importlib.util.spec_from_file_location('ref_datatools', ref_path)
-    ref = importlib.util.module_from_spec(spec); spec.loader.exec_module(ref)
+    """gru4rec_b200/datatools.py is an independent implementation; the reference's datatools.py was run on the same random
+    frames by oracle/make_standalone_golden.py (tests/golden/datatools_cases.json): same printed decision, same in-place
+    result, same int32 offsets."""
+    import json
+    from golden_utils import datatools_cases, datatools_outcome, GOLDEN_DIR
     from gru4rec_b200 import datatools as mine
-    rs = np.random.RandomState(0)
+    ref = json.load(open(os.path.join(GOLDEN_DIR, 'datatools_cases.json')))
     n_cases = 0
-    for n in (1, 2, 50, 300):
-        for trial in range(8):
-            df = pd.DataFrame({'SessionId': rs.randint(0, max(2, n // 4), n), 'Time': rs.randint(0, 40, n), 'ItemId': rs.randint(0, 9, n)})
-            if trial % 4 == 1: df = df.sort_values(['SessionId', 'Time']).reset_index(drop=True)
-            if trial % 4 == 2: df = df.sort_values(['SessionId', 'Time', 'ItemId']).reset_index(drop=True)
-            if trial % 4 == 3:      # sessions grouped but in arbitrary order
-                df = df.sort_values(['SessionId', 'Time']).reset_index(drop=True)
-                df = pd.concat([df[df.SessionId == s] for s in rs.permutation(df['SessionId'].unique())]).reset_index(drop=True)
-            for cols in (['SessionId', 'Time'], ['SessionId', 'Time', 'ItemId'], ['SessionId']):
-                for any_order in (False, True):
-                    a, b = df.copy(), df.copy()
-                    out_a, out_b = io.StringIO(), io.StringIO()
-                    with contextlib.redirect_stdout(out_a): ref.sort_if_needed(a, cols, any_order)
-                    with contextlib.redirect_stdout(out_b): mine.sort_if_needed(b, cols, any_order)
-                    keep = lambda t: [l for l in t.getvalue().splitlines() if not l.startswith('Data is sorted in')]
-                    assert keep(out_a) == keep(out_b)
-                    assert a.equals(b)
-                    oa, ob = ref.compute_offset(a, 'SessionId'), mine.compute_offset(b, 'SessionId')
-                    assert oa.dtype == ob.dtype and np.array_equal(oa, ob)
-                    n_cases += 1
-    assert n_cases == 192
+    for k, case in enumerate(datatools_cases()):
+        assert datatools_outcome(mine.sort_if_needed, mine.compute_offset, *case) == ref[k], (k, case[1:])
+        n_cases += 1
+    assert n_cases == len(ref) == 192
 
 
 def test_set_params_matches_the_reference_class():

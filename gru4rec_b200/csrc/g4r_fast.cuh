@@ -414,9 +414,10 @@ __device__ void fk_dense(const ModelDev& md, FastSmem& sm, int s, int cta) {
     for (int u = 0; u < U; u++) {
       if (!ok[u]) continue;
       float gs = g[u];
-      if (ada) { const float a = a0[u] + g[u] * g[u]; *pa[u] = a; gs = __fdiv_rn(g[u], sqrtf(a + G4R_EPS_ADA)); }
-      if (mom) { const float v2 = md.mom * v0[u] - md.lr * (gs + md.lmbd * p0[u]); *pv[u] = v2; *p[u] = p0[u] + v2; }
-      else *p[u] = p0[u] * (1.0f - md.lr * md.lmbd) - md.lr * gs;
+      if (ada) gs = adagrad_scale(g[u], a0[u], *pa[u]);
+      float v = v0[u];
+      *p[u] = dense_step(md, gs, p0[u], v, mom);
+      if (mom) *pv[u] = v;
     }
   }
 }
@@ -439,30 +440,13 @@ __device__ void fk_sparse_in(const ModelDev& md, SM& sm, int s, int b) {
   const bool ada = md.adapt == G4R_ADAPT_ADAGRAD, mom = md.mom > 0.f;
   float* prow = ly.Wx + (size_t)item * ld3;
   for (int c4 = tid; c4 < ld3 / 4; c4 += FK_THREADS) {
-    const float4 p0 = ld4(prow + c4 * 4);
-    float4 a0 = make_float4(0.f, 0.f, 0.f, 0.f), v0 = a0, al = a0, vl = a0;
-    if (ada) a0 = ld4(ly.Wx_acc + (size_t)item * ld3 + c4 * 4);
-    if (mom) v0 = ld4(ly.Wx_vel + (size_t)item * ld3 + c4 * 4);
-    float4 ps = p0;
-    for (int k = 0; k < nmem; k++) {
-      const float4 g = ld4(ly.dvec + (size_t)sm.gIdx[k] * ld3 + c4 * 4);
-      float4 gs = g;
-      if (ada) {
-        al.x = a0.x + g.x * g.x; al.y = a0.y + g.y * g.y; al.z = a0.z + g.z * g.z; al.w = a0.w + g.w * g.w;
-        gs.x = __fdiv_rn(g.x, sqrtf(al.x + G4R_EPS_ADA)); gs.y = __fdiv_rn(g.y, sqrtf(al.y + G4R_EPS_ADA));
-        gs.z = __fdiv_rn(g.z, sqrtf(al.z + G4R_EPS_ADA)); gs.w = __fdiv_rn(g.w, sqrtf(al.w + G4R_EPS_ADA));
-      }
-      float4 d;
-      if (md.lmbd > 0.f) { d.x = md.lr * (gs.x + md.lmbd * p0.x); d.y = md.lr * (gs.y + md.lmbd * p0.y); d.z = md.lr * (gs.z + md.lmbd * p0.z); d.w = md.lr * (gs.w + md.lmbd * p0.w); }
-      else { d.x = md.lr * gs.x; d.y = md.lr * gs.y; d.z = md.lr * gs.z; d.w = md.lr * gs.w; }
-      if (mom) {
-        vl.x = md.mom * v0.x - d.x; vl.y = md.mom * v0.y - d.y; vl.z = md.mom * v0.z - d.z; vl.w = md.mom * v0.w - d.w;
-        ps.x += vl.x; ps.y += vl.y; ps.z += vl.z; ps.w += vl.w;
-      } else { ps.x -= d.x; ps.y -= d.y; ps.z -= d.z; ps.w -= d.w; }
-    }
-    st4(prow + c4 * 4, ps);
-    if (ada) st4(ly.Wx_acc + (size_t)item * ld3 + c4 * 4, al);
-    if (mom) st4(ly.Wx_vel + (size_t)item * ld3 + c4 * 4, vl);
+    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+    SparseUpd4 u;
+    u.begin(ld4(prow + c4 * 4), ada ? ld4(ly.Wx_acc + (size_t)item * ld3 + c4 * 4) : z, mom ? ld4(ly.Wx_vel + (size_t)item * ld3 + c4 * 4) : z);
+    for (int k = 0; k < nmem; k++) u.add(md, ld4(ly.dvec + (size_t)sm.gIdx[k] * ld3 + c4 * 4), ada, mom);
+    st4(prow + c4 * 4, u.ps);
+    if (ada) st4(ly.Wx_acc + (size_t)item * ld3 + c4 * 4, u.al);
+    if (mom) st4(ly.Wx_vel + (size_t)item * ld3 + c4 * 4, u.vl);
   }
 }
 
@@ -493,26 +477,12 @@ __device__ void fk_sparse_in_one(const ModelDev& md, SM& sm, int s, int b, const
   __syncthreads();
   if (mine) {
     const int nmem = sm.gIdx[FK_B];
-    float4 al = a0, vl = v0, ps = p0;
-    for (int k = 0; k < nmem; k++) {
-      const float4 g = ld4(ly.dvec + (size_t)sm.gIdx[k] * ld3 + c4 * 4);
-      float4 gs = g;
-      if (ada) {
-        al.x = a0.x + g.x * g.x; al.y = a0.y + g.y * g.y; al.z = a0.z + g.z * g.z; al.w = a0.w + g.w * g.w;
-        gs.x = __fdiv_rn(g.x, sqrtf(al.x + G4R_EPS_ADA)); gs.y = __fdiv_rn(g.y, sqrtf(al.y + G4R_EPS_ADA));
-        gs.z = __fdiv_rn(g.z, sqrtf(al.z + G4R_EPS_ADA)); gs.w = __fdiv_rn(g.w, sqrtf(al.w + G4R_EPS_ADA));
-      }
-      float4 d;
-      if (md.lmbd > 0.f) { d.x = md.lr * (gs.x + md.lmbd * p0.x); d.y = md.lr * (gs.y + md.lmbd * p0.y); d.z = md.lr * (gs.z + md.lmbd * p0.z); d.w = md.lr * (gs.w + md.lmbd * p0.w); }
-      else { d.x = md.lr * gs.x; d.y = md.lr * gs.y; d.z = md.lr * gs.z; d.w = md.lr * gs.w; }
-      if (mom) {
-        vl.x = md.mom * v0.x - d.x; vl.y = md.mom * v0.y - d.y; vl.z = md.mom * v0.z - d.z; vl.w = md.mom * v0.w - d.w;
-        ps.x += vl.x; ps.y += vl.y; ps.z += vl.z; ps.w += vl.w;
-      } else { ps.x -= d.x; ps.y -= d.y; ps.z -= d.z; ps.w -= d.w; }
-    }
-    st4(prow + c4 * 4, ps);
-    if (ada) st4(ly.Wx_acc + (size_t)item * ld3 + c4 * 4, al);
-    if (mom) st4(ly.Wx_vel + (size_t)item * ld3 + c4 * 4, vl);
+    SparseUpd4 u;
+    u.begin(p0, a0, v0);
+    for (int k = 0; k < nmem; k++) u.add(md, ld4(ly.dvec + (size_t)sm.gIdx[k] * ld3 + c4 * 4), ada, mom);
+    st4(prow + c4 * 4, u.ps);
+    if (ada) st4(ly.Wx_acc + (size_t)item * ld3 + c4 * 4, u.al);
+    if (mom) st4(ly.Wx_vel + (size_t)item * ld3 + c4 * 4, u.vl);
   }
 }
 
@@ -831,7 +801,8 @@ __global__ void __launch_bounds__(FK_THREADS, 1) k_fast_t(int slot, int n_steps,
     }
     __syncthreads();
     FK_STAMP(13);
-    // sparse update from shared memory (rows prefetched before the step): one warp per duplicate group
+    // sparse update from shared memory (rows prefetched before the step): one warp per duplicate group.  Written out
+    // rather than with SparseUpd4 / SparseUpd, which cost this kernel a 16-byte register spill; same arithmetic.
     for (int j = warp; j < nj; j += FK_THREADS / 32) {
       const int item = sm.sIt[buf][j];
       if (j > 0 && sm.sIt[buf][j - 1] == item) continue;

@@ -375,9 +375,8 @@ __device__ void cf_backward(const ModelDev& md, FastSmemC& sm, const ClusterCtx&
       for (int e = 0; e < 4; e++) {
         const float g = ge[e], p0 = sm.rP[o + e];
         float gs = g;
-        if (ada) { const float a = sm.rA[o + e] + g * g; sm.rA[o + e] = a; gs = __fdiv_rn(g, sqrtf(a + G4R_EPS_ADA)); }
-        if (mom) { const float v2 = md.mom * sm.rV[o + e] - md.lr * (gs + md.lmbd * p0); sm.rV[o + e] = v2; sm.rP[o + e] = p0 + v2; }
-        else sm.rP[o + e] = p0 * (1.0f - md.lr * md.lmbd) - md.lr * gs;
+        if (ada) gs = adagrad_scale(g, sm.rA[o + e], sm.rA[o + e]);
+        sm.rP[o + e] = dense_step(md, gs, p0, sm.rV[o + e], mom);
       }
     }
   }
@@ -392,9 +391,8 @@ __device__ void cf_backward(const ModelDev& md, FastSmemC& sm, const ClusterCtx&
     const int o = lane * FC_PH + j;
     const float p0 = sm.rB[0][o];
     float gs = g;
-    if (ada) { const float a = sm.rB[1][o] + g * g; sm.rB[1][o] = a; gs = __fdiv_rn(g, sqrtf(a + G4R_EPS_ADA)); }
-    if (mom) { const float v2 = md.mom * sm.rB[2][o] - md.lr * (gs + md.lmbd * p0); sm.rB[2][o] = v2; sm.rB[0][o] = p0 + v2; }
-    else sm.rB[0][o] = p0 * (1.0f - md.lr * md.lmbd) - md.lr * gs;
+    if (ada) gs = adagrad_scale(g, sm.rB[1][o], sm.rB[1][o]);
+    sm.rB[0][o] = dense_step(md, gs, p0, sm.rB[2][o], mom);
   }
   __syncthreads();
   cl_arrive();          // this CTA no longer reads H*r of step s

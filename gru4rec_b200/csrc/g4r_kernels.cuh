@@ -324,8 +324,58 @@ __device__ __forceinline__ void stage_rows4(float* sdst, int sld, int nrows, int
   }
 }
 // ------------------------------------------------------------------------------------------------
+// The Adagrad(+momentum) update, written once: every kernel that trains calls these helpers (only the column role of
+// k_fast_t keeps an inline copy, which avoids a register spill there).  They take the gradient already scaled
+// (grad_scale).  The sparse and dense step tails are different formulas on purpose.
+// ------------------------------------------------------------------------------------------------
+// Adagrad scaling of one gradient against the OLD accumulator a0 (gru4rec.py:335-340): a = a0 + g^2, returns g / sqrt(a + eps)
+__device__ __forceinline__ float adagrad_scale(float g, float a0, float& a) {
+  a = a0 + g * g;
+  return __fdiv_rn(g, sqrtf(a + G4R_EPS_ADA));
+}
+// sparse step of one duplicate-group member (gru4rec.py:407-431): lmbd uses p0, the row before the update; the parameter
+// accumulates every member's step in ps, the velocity vl is the last member's
+__device__ __forceinline__ void sparse_step(const ModelDev& md, float gs, float p0, float v0, float& ps, float& vl, bool mom) {
+  const float d = md.lmbd > 0.f ? md.lr * (gs + md.lmbd * p0) : md.lr * gs;
+  if (mom) { vl = md.mom * v0 - d; ps += vl; } else ps -= d;
+}
+// dense step (gru4rec.py:390-406): returns the new parameter; v is the velocity, read and written only with momentum
+__device__ __forceinline__ float dense_step(const ModelDev& md, float gs, float p0, float& v, bool mom) {
+  if (mom) { v = md.mom * v - md.lr * (gs + md.lmbd * p0); return p0 + v; }
+  return p0 * (1.0f - md.lr * md.lmbd) - md.lr * gs;
+}
+// Adagrad(+momentum) of one element of an item row with the gradients of its duplicate group added in position order:
+// every member is scaled against the old accumulator a0, acc / velocity keep the last member's, the parameter accumulates
+struct SparseUpd {
+  float p0, a0, v0, ps, al, vl;
+  __device__ __forceinline__ void begin(float p, float a, float v) { p0 = p; a0 = a; v0 = v; ps = p; al = 0.f; vl = 0.f; }
+  __device__ __forceinline__ void add(const ModelDev& md, float g, bool ada, bool mom) {
+    sparse_step(md, ada ? adagrad_scale(g, a0, al) : g, p0, v0, ps, vl, mom);
+  }
+};
+// the same on a 16-byte quad of a row; plmbd is the row the lmbd term uses (the parameter row itself unless given).
+// One branch per condition covers all four components: written per component (SparseUpd::add four times), the compiler
+// turns the lmbd / mom branches into selects, which changes the FMA contraction of `ps -= d` and so the rounding.
+struct SparseUpd4 {
+  float4 p0, a0, v0, ps, al, vl;
+  __device__ __forceinline__ void begin(float4 p, float4 a, float4 v, float4 plmbd) { p0 = plmbd; a0 = a; v0 = v; ps = p; al = make_float4(0.f, 0.f, 0.f, 0.f); vl = al; }
+  __device__ __forceinline__ void begin(float4 p, float4 a, float4 v) { begin(p, a, v, p); }
+  __device__ __forceinline__ void add(const ModelDev& md, float4 g, bool ada, bool mom) {
+    if (ada) { g.x = adagrad_scale(g.x, a0.x, al.x); g.y = adagrad_scale(g.y, a0.y, al.y); g.z = adagrad_scale(g.z, a0.z, al.z); g.w = adagrad_scale(g.w, a0.w, al.w); }
+    float4 d;
+    if (md.lmbd > 0.f) { d.x = md.lr * (g.x + md.lmbd * p0.x); d.y = md.lr * (g.y + md.lmbd * p0.y); d.z = md.lr * (g.z + md.lmbd * p0.z); d.w = md.lr * (g.w + md.lmbd * p0.w); }
+    else { d.x = md.lr * g.x; d.y = md.lr * g.y; d.z = md.lr * g.z; d.w = md.lr * g.w; }
+    if (mom) {
+      vl.x = md.mom * v0.x - d.x; vl.y = md.mom * v0.y - d.y; vl.z = md.mom * v0.z - d.z; vl.w = md.mom * v0.w - d.w;
+      ps.x += vl.x; ps.y += vl.y; ps.z += vl.z; ps.w += vl.w;
+    } else { ps.x -= d.x; ps.y -= d.y; ps.z -= d.z; ps.w -= d.w; }
+  }
+};
+
+// ------------------------------------------------------------------------------------------------
 // Adaptive scalers other than Adagrad (gru4rec.py:300-329 adam, 341-366 adadelta, 367-381 rmsprop) and the update that follows
 // (gru4rec.py:390-431), for ONE element of a parameter with n gradient contributions in position order (n = 1: dense).
+// Only for adapt > G4R_ADAPT_ADAGRAD: Adagrad and plain SGD call the helpers above directly.
 // Sparse ("sampled") parameters use the reference's duplicate-accurate forms: the decayed state receives the squared
 // gradients of ALL duplicates, every duplicate is scaled with that common state (and adam's sparse first moment accumulates
 // grad**2 -- sic, gru4rec.py:325); velocity: last duplicate wins; parameter: all duplicates accumulate.
@@ -359,25 +409,17 @@ __device__ __forceinline__ void opt_elem(const ModelDev& md, OptE& e, float p0l,
     common = __fdiv_rn(__fdiv_rn(Mg, bias), sqrtf(__fdiv_rn(A, bias)) + G4R_EPS_ADA);
     e.s0 = A; e.s1 = Mg; e.s2 = ct;
   }
-  const float v0 = e.v, a0 = e.s0;
-  float ps = e.p, vl = e.v, al = e.s0;
+  const float v0 = e.v;
+  float ps = e.p, vl = e.v;
   for (int k = 0; k < n; k++) {
     const float g = gk(k) * gsc;
     float gs;
-    if (ad == G4R_ADAPT_ADAGRAD) { al = a0 + g * g; gs = __fdiv_rn(g, sqrtf(al + G4R_EPS_ADA)); }
-    else if (ad == G4R_ADAPT_RMSPROP) gs = g * sclr;
+    if (ad == G4R_ADAPT_RMSPROP) gs = g * sclr;
     else if (ad == G4R_ADAPT_ADADELTA) gs = g * sclr;
-    else if (ad == G4R_ADAPT_ADAM) gs = common;
-    else gs = g;
-    if (SPARSE) {
-      const float d = md.lmbd > 0.f ? md.lr * (gs + md.lmbd * p0l) : md.lr * gs;
-      if (mom) { vl = md.mom * v0 - d; ps += vl; } else ps -= d;
-    } else {
-      if (mom) { vl = md.mom * v0 - md.lr * (gs + md.lmbd * e.p); ps = e.p + vl; }
-      else ps = e.p * (1.0f - md.lr * md.lmbd) - md.lr * gs;
-    }
+    else gs = common;
+    if (SPARSE) sparse_step(md, gs, p0l, v0, ps, vl, mom);
+    else ps = dense_step(md, gs, e.p, vl, mom);         // dense: one member (n = 1), so vl is still v0 here
   }
-  if (ad == G4R_ADAPT_ADAGRAD) e.s0 = al;
   e.p = ps; e.v = vl;
 }
 // number of adaptive state arrays per parameter (they sit one after the other, `stride` elements apart, behind `*.acc`)
@@ -418,19 +460,11 @@ __device__ __forceinline__ void dense_update(const ModelDev& md, float* p, float
   }
   g *= grad_scale(md);
   float gs = g;
-  if (md.adapt == G4R_ADAPT_ADAGRAD) {
-    float a = *acc + g * g;
-    *acc = a;
-    gs = __fdiv_rn(g, sqrtf(a + G4R_EPS_ADA));
-  }
-  float pv = *p;
-  if (md.mom > 0.f) {
-    float v2 = md.mom * (*vel) - md.lr * (gs + md.lmbd * pv);
-    *vel = v2;
-    *p = pv + v2;
-  } else {
-    *p = pv * (1.0f - md.lr * md.lmbd) - md.lr * gs;
-  }
+  if (md.adapt == G4R_ADAPT_ADAGRAD) gs = adagrad_scale(g, *acc, *acc);
+  const bool mom = md.mom > 0.f;
+  float v = mom ? *vel : 0.f;
+  *p = dense_step(md, gs, *p, v, mom);
+  if (mom) *vel = v;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1033,31 +1067,17 @@ __device__ __forceinline__ void sparse_row_update(const ModelDev& md, float* __r
   }
   const float gsc = grad_scale(md);
   for (int c4 = lane; c4 < ld / 4; c4 += 32) {
-    const float4 p0 = ld4(prow + c4 * 4);
-    float4 a0 = make_float4(0.f, 0.f, 0.f, 0.f), v0 = a0, al = a0, vl = a0;
-    if (ada) a0 = ld4(arow + c4 * 4);
-    if (mom) v0 = ld4(vrow + c4 * 4);
-    float4 ps = p0;
+    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+    SparseUpd4 u;
+    u.begin(ld4(prow + c4 * 4), ada ? ld4(arow + c4 * 4) : z, mom ? ld4(vrow + c4 * 4) : z);
     for (int k = 0; k < n_members; k++) {
       float4 g = ld4(gsrc + (size_t)k * gstride + c4 * 4);
       g.x *= gsc; g.y *= gsc; g.z *= gsc; g.w *= gsc;
-      float4 gs = g;
-      if (ada) {
-        al.x = a0.x + g.x * g.x; al.y = a0.y + g.y * g.y; al.z = a0.z + g.z * g.z; al.w = a0.w + g.w * g.w;
-        gs.x = __fdiv_rn(g.x, sqrtf(al.x + G4R_EPS_ADA)); gs.y = __fdiv_rn(g.y, sqrtf(al.y + G4R_EPS_ADA));
-        gs.z = __fdiv_rn(g.z, sqrtf(al.z + G4R_EPS_ADA)); gs.w = __fdiv_rn(g.w, sqrtf(al.w + G4R_EPS_ADA));
-      }
-      float4 d;
-      if (md.lmbd > 0.f) { d.x = md.lr * (gs.x + md.lmbd * p0.x); d.y = md.lr * (gs.y + md.lmbd * p0.y); d.z = md.lr * (gs.z + md.lmbd * p0.z); d.w = md.lr * (gs.w + md.lmbd * p0.w); }
-      else { d.x = md.lr * gs.x; d.y = md.lr * gs.y; d.z = md.lr * gs.z; d.w = md.lr * gs.w; }
-      if (mom) {
-        vl.x = md.mom * v0.x - d.x; vl.y = md.mom * v0.y - d.y; vl.z = md.mom * v0.z - d.z; vl.w = md.mom * v0.w - d.w;
-        ps.x += vl.x; ps.y += vl.y; ps.z += vl.z; ps.w += vl.w;
-      } else { ps.x -= d.x; ps.y -= d.y; ps.z -= d.z; ps.w -= d.w; }
+      u.add(md, g, ada, mom);
     }
-    st4(prow + c4 * 4, ps);
-    if (ada) st4(arow + c4 * 4, al);
-    if (mom) st4(vrow + c4 * 4, vl);
+    st4(prow + c4 * 4, u.ps);
+    if (ada) st4(arow + c4 * 4, u.al);
+    if (mom) st4(vrow + c4 * 4, u.vl);
   }
 }
 
@@ -1083,18 +1103,12 @@ __device__ __forceinline__ void chunk_rows_update(const ModelDev& md, const int*
                                      [&](int k, int) { return gDby[j - gDoff + k]; });
     } else if (lane == 0) {   // By (gru4rec.py:486-489)
       const float gsc = grad_scale(md);
-      const float p0 = md.By[item];
-      float a0 = ada ? md.By_acc[item] : 0.f, v0 = mom ? md.By_vel[item] : 0.f, al = 0.f, vl = 0.f, ps = p0;
-      for (int jj = j; jj < je; jj++) {
-        const float g = gDby[jj - gDoff] * gsc;
-        float gs = g;
-        if (ada) { al = a0 + g * g; gs = __fdiv_rn(g, sqrtf(al + G4R_EPS_ADA)); }
-        const float d = md.lmbd > 0.f ? md.lr * (gs + md.lmbd * p0) : md.lr * gs;
-        if (mom) { vl = md.mom * v0 - d; ps += vl; } else ps -= d;
-      }
-      md.By[item] = ps;
-      if (ada) md.By_acc[item] = al;
-      if (mom) md.By_vel[item] = vl;
+      SparseUpd u;
+      u.begin(md.By[item], ada ? md.By_acc[item] : 0.f, mom ? md.By_vel[item] : 0.f);
+      for (int jj = j; jj < je; jj++) u.add(md, gDby[jj - gDoff] * gsc, ada, mom);
+      md.By[item] = u.ps;
+      if (ada) md.By_acc[item] = u.al;
+      if (mom) md.By_vel[item] = u.vl;
     }
   }
 }
@@ -1445,7 +1459,7 @@ __device__ void phase_sparse_in(const ModelDev& md, int s, int b, bool apply_pas
   const float gsc = grad_scale(md);
   for (int c4 = threadIdx.x; c4 < ld / 4; c4 += blockDim.x) {
     const float4 pcur = ld4(prow + c4 * 4);
-    float4 a0 = make_float4(0.f, 0.f, 0.f, 0.f), v0 = a0, al = a0, vl = a0, p0 = pcur;
+    float4 a0 = make_float4(0.f, 0.f, 0.f, 0.f), v0 = a0, p0 = pcur;
     if (shared) {
       p0 = ld4(md.Sx + (size_t)b * ldg + c4 * 4);         // row value before the Wy update (sparam)
       if (ada) a0 = ld4(md.snapAcc + (size_t)b * ldg + c4 * 4);
@@ -1454,28 +1468,17 @@ __device__ void phase_sparse_in(const ModelDev& md, int s, int b, bool apply_pas
       if (ada) a0 = ld4(tacc + (size_t)item * ld + c4 * 4);
       if (mom) v0 = ld4(tvel + (size_t)item * ld + c4 * 4);
     }
-    float4 ps = pcur;
+    SparseUpd4 u;
+    u.begin(pcur, a0, v0, p0);
     for (int bb = b; bb >= 0; bb = xnext[bb]) {
       float4 g = ld4(G + (size_t)bb * ldg + c4 * 4);
       g.x *= gsc; g.y *= gsc; g.z *= gsc; g.w *= gsc;
-      float4 gs = g;
-      if (ada) {
-        al.x = a0.x + g.x * g.x; al.y = a0.y + g.y * g.y; al.z = a0.z + g.z * g.z; al.w = a0.w + g.w * g.w;
-        gs.x = __fdiv_rn(g.x, sqrtf(al.x + G4R_EPS_ADA)); gs.y = __fdiv_rn(g.y, sqrtf(al.y + G4R_EPS_ADA));
-        gs.z = __fdiv_rn(g.z, sqrtf(al.z + G4R_EPS_ADA)); gs.w = __fdiv_rn(g.w, sqrtf(al.w + G4R_EPS_ADA));
-      }
-      float4 d;
-      if (md.lmbd > 0.f) { d.x = md.lr * (gs.x + md.lmbd * p0.x); d.y = md.lr * (gs.y + md.lmbd * p0.y); d.z = md.lr * (gs.z + md.lmbd * p0.z); d.w = md.lr * (gs.w + md.lmbd * p0.w); }
-      else { d.x = md.lr * gs.x; d.y = md.lr * gs.y; d.z = md.lr * gs.z; d.w = md.lr * gs.w; }
-      if (mom) {
-        vl.x = md.mom * v0.x - d.x; vl.y = md.mom * v0.y - d.y; vl.z = md.mom * v0.z - d.z; vl.w = md.mom * v0.w - d.w;
-        ps.x += vl.x; ps.y += vl.y; ps.z += vl.z; ps.w += vl.w;
-      } else { ps.x -= d.x; ps.y -= d.y; ps.z -= d.z; ps.w -= d.w; }
+      u.add(md, g, ada, mom);
     }
-    st4(prow + c4 * 4, ps);
+    st4(prow + c4 * 4, u.ps);
     if (write_state) {
-      if (ada) st4(tacc + (size_t)item * ld + c4 * 4, al);
-      if (mom) st4(tvel + (size_t)item * ld + c4 * 4, vl);
+      if (ada) st4(tacc + (size_t)item * ld + c4 * 4, u.al);
+      if (mom) st4(tvel + (size_t)item * ld + c4 * 4, u.vl);
     }
   }
 }

@@ -133,31 +133,16 @@ __global__ void __launch_bounds__(256) k_mg_plan2(ModelDev md, MgDev mg, int n_s
 __device__ __forceinline__ void mg_row_update(const ModelDev& md, float* prow, float* arow, float* vrow, const int* ent, int n, int shift, int mask,
                                               const float* gbase, size_t rstride, int gld, int lane, int ld, bool ada, bool mom) {
   for (int c4 = lane; c4 < ld / 4; c4 += 32) {
-    const float4 p0 = ld4(prow + c4 * 4);
-    float4 a0 = make_float4(0.f, 0.f, 0.f, 0.f), v0 = a0, al = a0, vl = a0;
-    if (ada) a0 = ld4(arow + c4 * 4);
-    if (mom) v0 = ld4(vrow + c4 * 4);
-    float4 ps = p0;
+    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+    SparseUpd4 u;
+    u.begin(ld4(prow + c4 * 4), ada ? ld4(arow + c4 * 4) : z, mom ? ld4(vrow + c4 * 4) : z);
     for (int k = 0; k < n; k++) {
       const int e = ent[k];
-      const float4 g = ld4(gbase + ((size_t)(e >> shift) * rstride + (size_t)(e & mask)) * gld + c4 * 4);
-      float4 gs = g;
-      if (ada) {
-        al.x = a0.x + g.x * g.x; al.y = a0.y + g.y * g.y; al.z = a0.z + g.z * g.z; al.w = a0.w + g.w * g.w;
-        gs.x = __fdiv_rn(g.x, sqrtf(al.x + G4R_EPS_ADA)); gs.y = __fdiv_rn(g.y, sqrtf(al.y + G4R_EPS_ADA));
-        gs.z = __fdiv_rn(g.z, sqrtf(al.z + G4R_EPS_ADA)); gs.w = __fdiv_rn(g.w, sqrtf(al.w + G4R_EPS_ADA));
-      }
-      float4 d;
-      if (md.lmbd > 0.f) { d.x = md.lr * (gs.x + md.lmbd * p0.x); d.y = md.lr * (gs.y + md.lmbd * p0.y); d.z = md.lr * (gs.z + md.lmbd * p0.z); d.w = md.lr * (gs.w + md.lmbd * p0.w); }
-      else { d.x = md.lr * gs.x; d.y = md.lr * gs.y; d.z = md.lr * gs.z; d.w = md.lr * gs.w; }
-      if (mom) {
-        vl.x = md.mom * v0.x - d.x; vl.y = md.mom * v0.y - d.y; vl.z = md.mom * v0.z - d.z; vl.w = md.mom * v0.w - d.w;
-        ps.x += vl.x; ps.y += vl.y; ps.z += vl.z; ps.w += vl.w;
-      } else { ps.x -= d.x; ps.y -= d.y; ps.z -= d.z; ps.w -= d.w; }
+      u.add(md, ld4(gbase + ((size_t)(e >> shift) * rstride + (size_t)(e & mask)) * gld + c4 * 4), ada, mom);
     }
-    st4(prow + c4 * 4, ps);
-    if (ada) st4(arow + c4 * 4, al);
-    if (mom) st4(vrow + c4 * 4, vl);
+    st4(prow + c4 * 4, u.ps);
+    if (ada) st4(arow + c4 * 4, u.al);
+    if (mom) st4(vrow + c4 * 4, u.vl);
   }
 }
 
@@ -179,19 +164,15 @@ __global__ void __launch_bounds__(256) k_mg_apply_rows(int slot, MgDev mg, const
     mg_row_update(md, md.Wy + (size_t)item * md.ldL, md.Wy_acc ? md.Wy_acc + (size_t)item * md.ldL : nullptr, md.Wy_vel ? md.Wy_vel + (size_t)item * md.ldL : nullptr,
                   ent + j, je - j, 20, 0xfffff, mg.DSYall, (size_t)md.NP, md.ldL, lane, md.ldL, ada, mom);
     if (lane == 0) {
-      const float p0 = md.By[item];
-      float a0 = ada ? md.By_acc[item] : 0.f, v0 = mom ? md.By_vel[item] : 0.f, al = 0.f, vl = 0.f, ps = p0;
+      SparseUpd u;
+      u.begin(md.By[item], ada ? md.By_acc[item] : 0.f, mom ? md.By_vel[item] : 0.f);
       for (int k = j; k < je; k++) {
         const int e = ent[k];
-        const float g = mg.DBYall[(size_t)(e >> 20) * md.NP + (e & 0xfffff)];
-        float gs = g;
-        if (ada) { al = a0 + g * g; gs = __fdiv_rn(g, sqrtf(al + G4R_EPS_ADA)); }
-        const float d = md.lmbd > 0.f ? md.lr * (gs + md.lmbd * p0) : md.lr * gs;
-        if (mom) { vl = md.mom * v0 - d; ps += vl; } else ps -= d;
+        u.add(md, mg.DBYall[(size_t)(e >> 20) * md.NP + (e & 0xfffff)], ada, mom);
       }
-      md.By[item] = ps;
-      if (ada) md.By_acc[item] = al;
-      if (mom) md.By_vel[item] = vl;
+      md.By[item] = u.ps;
+      if (ada) md.By_acc[item] = u.al;
+      if (mom) md.By_vel[item] = u.vl;
     }
   }
 }
@@ -215,38 +196,17 @@ __global__ void __launch_bounds__(128) k_mg_apply_in(int slot, MgDev mg, const i
   const int lane = threadIdx.x;        // all 128 threads stride over the 16-byte columns of the row
   for (int c4 = lane; c4 < ld / 4; c4 += 128) {
     float* prow = tab + (size_t)item * ld;
-    const float4 p0 = ld4(prow + c4 * 4);
-    float4 a0 = make_float4(0.f, 0.f, 0.f, 0.f), v0 = a0, al = a0, vl = a0;
-    if (ada) a0 = ld4(tacc + (size_t)item * ld + c4 * 4);
-    if (mom) v0 = ld4(tvel + (size_t)item * ld + c4 * 4);
-    float4 ps = p0;
+    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+    SparseUpd4 u;
+    u.begin(ld4(prow + c4 * 4), ada ? ld4(tacc + (size_t)item * ld + c4 * 4) : z, mom ? ld4(tvel + (size_t)item * ld + c4 * 4) : z);
     for (int k = j; k < je; k++) {
       const int e = ent[k];
-      const float4 g = ld4(mg.INall + ((size_t)(e >> 16) * md.B + (size_t)(e & 0xffff)) * ld + c4 * 4);
-      float4 gs = g;
-      if (ada) {
-        al.x = a0.x + g.x * g.x; al.y = a0.y + g.y * g.y; al.z = a0.z + g.z * g.z; al.w = a0.w + g.w * g.w;
-        gs.x = __fdiv_rn(g.x, sqrtf(al.x + G4R_EPS_ADA)); gs.y = __fdiv_rn(g.y, sqrtf(al.y + G4R_EPS_ADA));
-        gs.z = __fdiv_rn(g.z, sqrtf(al.z + G4R_EPS_ADA)); gs.w = __fdiv_rn(g.w, sqrtf(al.w + G4R_EPS_ADA));
-      }
-      float4 d;
-      if (md.lmbd > 0.f) { d.x = md.lr * (gs.x + md.lmbd * p0.x); d.y = md.lr * (gs.y + md.lmbd * p0.y); d.z = md.lr * (gs.z + md.lmbd * p0.z); d.w = md.lr * (gs.w + md.lmbd * p0.w); }
-      else { d.x = md.lr * gs.x; d.y = md.lr * gs.y; d.z = md.lr * gs.z; d.w = md.lr * gs.w; }
-      if (mom) {
-        vl.x = md.mom * v0.x - d.x; vl.y = md.mom * v0.y - d.y; vl.z = md.mom * v0.z - d.z; vl.w = md.mom * v0.w - d.w;
-        ps.x += vl.x; ps.y += vl.y; ps.z += vl.z; ps.w += vl.w;
-      } else { ps.x -= d.x; ps.y -= d.y; ps.z -= d.z; ps.w -= d.w; }
+      u.add(md, ld4(mg.INall + ((size_t)(e >> 16) * md.B + (size_t)(e & 0xffff)) * ld + c4 * 4), ada, mom);
     }
-    st4(prow + c4 * 4, ps);
-    if (ada) st4(tacc + (size_t)item * ld + c4 * 4, al);
-    if (mom) st4(tvel + (size_t)item * ld + c4 * 4, vl);
+    st4(prow + c4 * 4, u.ps);
+    if (ada) st4(tacc + (size_t)item * ld + c4 * 4, u.al);
+    if (mom) st4(tvel + (size_t)item * ld + c4 * 4, u.vl);
   }
-}
-// dense update from the all-reduced gradient of one tensor
-__global__ void __launch_bounds__(256) k_mg_apply_dense(int slot, float* p, float* acc, float* vel, const float* g, int n) {
-  const ModelDev& md = MD;
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) dense_update(md, p + i, acc ? acc + i : nullptr, vel ? vel + i : nullptr, g[i]);
 }
 
 struct MgHost {
@@ -329,7 +289,7 @@ static int mg_run_window(g4r_handle* h, int64_t n) {
     NC(g_nccl.GroupEnd());
     k_mg_apply_rows<<<md.NCH, 256, 0, st>>>(h->slot, mg, base, off);
     k_mg_apply_in<<<R * B, 128, 0, st>>>(h->slot, mg, base, off);
-    for (const MgTensor& t : tens) k_mg_apply_dense<<<(t.count + 255) / 256, 256, 0, st>>>(h->slot, t.p, t.acc, t.vel, mg.gradFlat + t.goff, t.count);
+    for (const MgTensor& t : tens) k_apply_dense<<<(t.count + 255) / 256, 256, 0, st>>>(h->slot, t.p, t.acc, t.vel, mg.gradFlat + t.goff, t.count);
     h->launches += 2 + (int64_t)tens.size();
     return G4R_OK;
   };

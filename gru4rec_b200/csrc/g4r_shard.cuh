@@ -163,27 +163,6 @@ __device__ __forceinline__ void fk_prefetch_mg(const ModelDev& md, FastSmemMG& s
   }
 }
 
-// Adagrad(+momentum) of one 16-byte quad with `n` gradient quads applied in order (gru4rec.py:335-340,407-431)
-struct QuadUpd {
-  float4 p0, a0, v0, al, vl, ps;
-  __device__ __forceinline__ void begin(float4 p, float4 a, float4 v) { p0 = p; a0 = a; v0 = v; al = a; vl = v; ps = p; }
-  __device__ __forceinline__ void add(const ModelDev& md, float4 g, bool ada, bool mom) {
-    float4 gs = g;
-    if (ada) {
-      al.x = a0.x + g.x * g.x; al.y = a0.y + g.y * g.y; al.z = a0.z + g.z * g.z; al.w = a0.w + g.w * g.w;
-      gs.x = __fdiv_rn(g.x, sqrtf(al.x + G4R_EPS_ADA)); gs.y = __fdiv_rn(g.y, sqrtf(al.y + G4R_EPS_ADA));
-      gs.z = __fdiv_rn(g.z, sqrtf(al.z + G4R_EPS_ADA)); gs.w = __fdiv_rn(g.w, sqrtf(al.w + G4R_EPS_ADA));
-    }
-    float4 d;
-    if (md.lmbd > 0.f) { d.x = md.lr * (gs.x + md.lmbd * p0.x); d.y = md.lr * (gs.y + md.lmbd * p0.y); d.z = md.lr * (gs.z + md.lmbd * p0.z); d.w = md.lr * (gs.w + md.lmbd * p0.w); }
-    else { d.x = md.lr * gs.x; d.y = md.lr * gs.y; d.z = md.lr * gs.z; d.w = md.lr * gs.w; }
-    if (mom) {
-      vl.x = md.mom * v0.x - d.x; vl.y = md.mom * v0.y - d.y; vl.z = md.mom * v0.z - d.z; vl.w = md.mom * v0.w - d.w;
-      ps.x += vl.x; ps.y += vl.y; ps.z += vl.z; ps.w += vl.w;
-    } else { ps.x -= d.x; ps.y -= d.y; ps.z -= d.z; ps.w -= d.w; }
-  }
-};
-
 // owner side: merged update of the rows of apply-chunk `a` (one warp per item group, members in (rank, position) order)
 __device__ void mgs_apply_rows(const ModelDev& md, FastSmemMG& sm, int s, int a, int par, unsigned int T) {
   const ShardDev& sh = sm.sh;
@@ -204,7 +183,7 @@ __device__ void mgs_apply_rows(const ModelDev& md, FastSmemMG& sm, int s, int a,
     const size_t ro = (size_t)(item / R) * ldW;
     for (int q4 = lane; q4 < nq; q4 += 32) {
       const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-      QuadUpd u;
+      SparseUpd4 u;
       u.begin(ld4(W + ro + q4 * 4), ada ? ld4(sh.W_acc + ro + q4 * 4) : z, mom ? ld4(sh.W_vel + ro + q4 * 4) : z);
       for (int k = j; k < je; k++) {
         const int e = ent[k];
@@ -235,7 +214,7 @@ __device__ void mgs_apply_inputs(const ModelDev& md, FastSmemMG& sm, int s, int 
     const size_t ro = (size_t)(item / R) * ld3;
     for (int q4 = tid; q4 < ld3 / 4; q4 += FK_THREADS) {
       const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-      QuadUpd u;
+      SparseUpd4 u;
       u.begin(ld4(Tb + ro + q4 * 4), ada ? ld4(sh.Wx_acc + ro + q4 * 4) : z, mom ? ld4(sh.Wx_vel + ro + q4 * 4) : z);
       for (int k = j; k < je; k++) {
         const int e = ent[k];
@@ -350,9 +329,10 @@ __device__ void fk_dense_mg(const ModelDev& md, FastSmemMG& sm, int s, int cta, 
     else { const int c = cb0 + (o - nWh - nWrz); p = ly.Bh + c; pa = ly.Bh_acc ? ly.Bh_acc + c : nullptr; pv = ly.Bh_vel ? ly.Bh_vel + c : nullptr; }
     const float p0 = *p;
     float gs = g;
-    if (ada) { const float a = *pa + g * g; *pa = a; gs = __fdiv_rn(g, sqrtf(a + G4R_EPS_ADA)); }
-    if (mom) { const float v2 = md.mom * (*pv) - md.lr * (gs + md.lmbd * p0); *pv = v2; *p = p0 + v2; }
-    else *p = p0 * (1.0f - md.lr * md.lmbd) - md.lr * gs;
+    if (ada) gs = adagrad_scale(g, *pa, *pa);
+    float v = mom ? *pv : 0.f;
+    *p = dense_step(md, gs, p0, v, mom);
+    if (mom) *pv = v;
   }
 }
 

@@ -42,6 +42,7 @@ EXPORTS = [
     'g4r_profile_uploaded', 'g4r_phase_name', 'g4r_phase_count', 'g4r_persistent_stamps', 'g4r_fast_windows', 'g4r_uses_tensor_cores', 'g4r_mg_unique_id', 'g4r_mg_init',
     'g4r_mg_sharded', 'g4r_mg_ipc_handle', 'g4r_mg_ipc_open', 'g4r_mg_owner', 'g4r_mg_local_row', 'g4r_mg_shard_rows', 'g4r_mg_segment_bytes',
     'g4r_eval_schedule', 'g4r_set_eval_items', 'g4r_predict', 'g4r_reset_eval_hidden',
+    'g4r_predict_topk',
 ]
 
 _lib = None
@@ -108,6 +109,7 @@ def load():
     lib.g4r_set_eval_items.argtypes = [vp, vp, i64]
     lib.g4r_predict.argtypes = [vp, vp, i32, vp, vp]
     lib.g4r_reset_eval_hidden.argtypes = [vp]
+    lib.g4r_predict_topk.argtypes = [vp, vp, i32, vp, vp, i64, i32, vp, vp]
     _lib = lib
     return lib
 
@@ -482,6 +484,21 @@ class Engine(object):
         out = np.empty((len(X), self.cfg.n_items), dtype=np.float32)
         self._check(self.lib.g4r_predict(self.h, _ptr(X), len(X), _ptr(rm), _ptr(out)))
         return out
+
+    def predict_topk(self, X, k, reset_mask=None, cand=None):
+        """The k best items of each lane among the scores predict() would return for the same call (the scoring-path hidden state
+        advances the same way), selected on the device.  cand: optional item indices (no duplicates) the items compete among;
+        softmax-family scores are then normalised over them.  Returns (items int32 [batch, k], scores float32 [batch, k]), each row
+        by score descending, ties by item index ascending."""
+        X = np.ascontiguousarray(X, dtype=np.int32)
+        rm = None if reset_mask is None else np.ascontiguousarray(reset_mask, dtype=np.uint8)
+        cd = None if cand is None else np.ascontiguousarray(cand, dtype=np.int64)
+        k = int(k)
+        items = np.empty((len(X), max(k, 0)), dtype=np.int32)
+        scores = np.empty((len(X), max(k, 0)), dtype=np.float32)
+        self._check(self.lib.g4r_predict_topk(self.h, _ptr(X), len(X), _ptr(rm), _ptr(cd), 0 if cd is None else cd.size, k,
+                                              _ptr(items), _ptr(scores)))
+        return items, scores
 
     def reset_eval_hidden(self):
         self._check(self.lib.g4r_reset_eval_hidden(self.h))

@@ -11,6 +11,8 @@ constexpr int EV_KT = 128;    // feature slab
 constexpr int EV_LDS = EV_KT + 4;
 constexpr int EV_THREADS = 256;
 
+#include "g4r_topk.cuh"
+
 // mode 'tiebreaking' (evaluation.py:55,65): yhat += U(0,1) * 1e-10 before the standard ranking.  The reference draws the noise
 // from Theano's MRG stream (not reproducible offline); here it is a counter hash of (evaluation step, lane, score column), so
 // the target's own column carries the same noise in the target score and in the tile and never beats itself.
@@ -205,6 +207,13 @@ struct EvalCtx {
   int slot = -1;
   int* dCand = nullptr; int n_cand = 0; size_t cand_cap = 0;     // candidate subset of evaluate_gpu(items=...), item indices
   unsigned char *dAsplit = nullptr, *dBsplit = nullptr;           // tcgen05 path: hi / lo TF32 operand blocks (g4r_eval_tc.cuh)
+  // g4r_predict_topk (g4r_topk.cuh): its own candidate list (the evaluation subset above is left alone), the per-partition lists,
+  // the results, and per k the lane-buffer size and CTAs per SM of k_topk_score (0 = not yet computed)
+  int* dTkCand = nullptr; size_t tk_cand_cap = 0;
+  float* dTkK = nullptr; int* dTkI = nullptr; size_t tk_part_cap = 0;
+  float* dTkMZ = nullptr; size_t tk_mz_cap = 0;
+  int* dTkItems = nullptr; float* dTkScores = nullptr; size_t tk_out_cap = 0;
+  int tk_cap[TK_MAX_K + 1] = {}, tk_occ[TK_MAX_K + 1] = {};
 };
 
 static void eval_release(g4r_handle* h) {
@@ -214,6 +223,7 @@ static void eval_release(g4r_handle* h) {
   cudaFree(e.dX); cudaFree(e.dY); cudaFree(e.dSlot); cudaFree(e.dF); cudaFree(e.dM); cudaFree(e.dSti); cudaFree(e.dG);
   cudaFree(e.dCut); cudaFree(e.dSums); if (e.dOut) cudaFree(e.dOut); if (e.dCand) cudaFree(e.dCand);
   if (e.dAsplit) cudaFree(e.dAsplit); if (e.dBsplit) cudaFree(e.dBsplit);
+  cudaFree(e.dTkCand); cudaFree(e.dTkK); cudaFree(e.dTkI); cudaFree(e.dTkMZ); cudaFree(e.dTkItems); cudaFree(e.dTkScores);
   slot_free(e.slot);
   delete static_cast<EvalCtx*>(h->eval_ctx);
   h->eval_ctx = nullptr;
@@ -238,6 +248,9 @@ static int eval_ctx(g4r_handle* h, EvalCtx** out) {
   CK(slot_upload(e.slot, e.mde, h->stream));
   cudaFuncSetAttribute(k_eval_score<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)eval_smem_bytes());
   cudaFuncSetAttribute(k_eval_score<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)eval_smem_bytes());
+  int smem_optin = 0;       // k_topk_score: its lane buffers may take all the shared memory a CTA can have (topk_shape)
+  if (cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->cfg.device) != cudaSuccess ||
+      cudaFuncSetAttribute(k_topk_score, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin) != cudaSuccess) cudaGetLastError();
   if (cudaFuncSetAttribute(k_eval_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TcSmem)) != cudaSuccess) cudaGetLastError();
   h->eval_ctx = new EvalCtx(e);
   *out = static_cast<EvalCtx*>(h->eval_ctx);
@@ -398,6 +411,99 @@ extern "C" int g4r_predict(g4r_handle* h, const int32_t* X, int32_t batch, const
   h->launches += 2;
   CK(cudaGetLastError());
   CK(cudaMemcpyAsync(out, e->dOut, need * sizeof(float), cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  return G4R_OK;
+}
+
+// Lane-buffer size of k_topk_score for this k: k + one tile at least, grown by whole tiles while the CTAs per SM stay the same
+// (more slack = fewer cuts of the buffers).  Partitions of the catalogue per lane block: enough CTAs to fill the SMs once.
+static int topk_shape(g4r_handle* h, EvalCtx* e, int k, int* cap, int* occ) {
+  if (!e->tk_cap[k]) {
+    int smem_optin = 0, o1 = 0;
+    CK(cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->cfg.device));
+    int c = k + EV_IT;
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o1, k_topk_score, EV_THREADS, topk_score_smem_bytes(c)));
+    if (o1 < 1) FAIL(G4R_ERR_CUDA, "k_topk_score does not fit on a multiprocessor");
+    for (int more = 0; more < 16; more++) {
+      const size_t sm = topk_score_smem_bytes(c + EV_IT);
+      int o = 0;
+      if (sm > (size_t)smem_optin) break;
+      CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, k_topk_score, EV_THREADS, sm));
+      if (o < o1) break;
+      c += EV_IT;
+    }
+    e->tk_cap[k] = c; e->tk_occ[k] = o1;
+  }
+  *cap = e->tk_cap[k]; *occ = e->tk_occ[k];
+  return G4R_OK;
+}
+
+extern "C" int g4r_predict_topk(g4r_handle* h, const int32_t* X, int32_t batch, const uint8_t* reset_mask,
+                                const int64_t* cand, int64_t n_cand, int32_t k, int32_t* items_out, float* scores_out) {
+  if (!h || !X || !items_out || !scores_out || n_cand < 0 || (n_cand > 0 && !cand)) return G4R_ERR_INVALID;
+  cudaSetDevice(h->cfg.device);
+  EvalCtx* e = nullptr;
+  int rc = eval_ctx(h, &e);
+  if (rc) return rc;
+  const int Be = e->Be, I = h->md.n_items;
+  if (batch <= 0 || batch > Be) FAIL(G4R_ERR_INVALID, "predict batch exceeds eval_batch_size");
+  if (n_cand > (int64_t)1 << 30) FAIL(G4R_ERR_INVALID, "too many candidate items");
+  const int n_comp = n_cand > 0 ? (int)n_cand : I;
+  if (k < 1 || k > TK_MAX_K || k > n_comp) FAIL(G4R_ERR_INVALID, "k must be in 1 .. min(256, number of candidate items)");
+  for (int b = 0; b < batch; b++)
+    if (X[b] < 0 || X[b] >= I) FAIL(G4R_ERR_INDEX, "Index out of bounds");
+  cudaStream_t st = h->stream;
+  if (n_cand > 0) {
+    std::vector<int> tmp((size_t)n_cand);
+    for (int64_t i = 0; i < n_cand; i++) {
+      if (cand[i] < 0 || cand[i] >= I) FAIL(G4R_ERR_INDEX, "Index out of bounds");
+      tmp[(size_t)i] = (int)cand[i];
+    }
+    std::vector<uint8_t> seen((size_t)I, 0);
+    for (const int c : tmp) {
+      if (seen[c]) FAIL(G4R_ERR_INVALID, "duplicate candidate item");
+      seen[c] = 1;
+    }
+    if (e->tk_cand_cap < (size_t)n_cand) { cudaFree(e->dTkCand); e->dTkCand = nullptr; e->tk_cand_cap = 0; CK(cudaMalloc(&e->dTkCand, (size_t)n_cand * sizeof(int))); e->tk_cand_cap = (size_t)n_cand; }
+    CK(cudaMemcpyAsync(e->dTkCand, tmp.data(), (size_t)n_cand * sizeof(int), cudaMemcpyHostToDevice, st));
+  }
+  int cap = 0, occ = 0;
+  rc = topk_shape(h, e, k, &cap, &occ);
+  if (rc) return rc;
+  const int lblocks = (batch + EV_TB - 1) / EV_TB, tiles = (n_comp + EV_IT - 1) / EV_IT;
+  // one wave of CTAs; each partition at least one tile; at most 16384 partial entries per lane for the merge
+  const int parts = std::max(1, std::min({h->n_sm * occ / lblocks, tiles, 16384 / k}));
+  const size_t n_part = (size_t)batch * parts * k, n_mz = (size_t)batch * parts * 2, n_out = (size_t)batch * k;
+  if (e->tk_part_cap < n_part) {
+    cudaFree(e->dTkK); cudaFree(e->dTkI); e->dTkK = nullptr; e->dTkI = nullptr; e->tk_part_cap = 0;
+    CK(cudaMalloc(&e->dTkK, n_part * sizeof(float))); CK(cudaMalloc(&e->dTkI, n_part * sizeof(int))); e->tk_part_cap = n_part;
+  }
+  if (e->tk_mz_cap < n_mz) { cudaFree(e->dTkMZ); e->dTkMZ = nullptr; e->tk_mz_cap = 0; CK(cudaMalloc(&e->dTkMZ, n_mz * sizeof(float))); e->tk_mz_cap = n_mz; }
+  if (e->tk_out_cap < n_out) {
+    cudaFree(e->dTkItems); cudaFree(e->dTkScores); e->dTkItems = nullptr; e->dTkScores = nullptr; e->tk_out_cap = 0;
+    CK(cudaMalloc(&e->dTkItems, n_out * sizeof(int))); CK(cudaMalloc(&e->dTkScores, n_out * sizeof(float))); e->tk_out_cap = n_out;
+  }
+  // lanes staged exactly as g4r_predict stages them: one event per lane, reset_mask -> flag 2 (zero the lane first)
+  for (int b = 0; b < Be; b++) {
+    e->hX[b] = b < batch ? X[b] : -1; e->hY[b] = 0; e->hSlot[b] = b;
+    e->hF[b] = (b < batch && reset_mask && reset_mask[b]) ? 2 : 0;
+  }
+  e->hM[0] = batch; e->hSti[0] = -1; e->hG[0] = 0;
+  CK(cudaMemcpyAsync(e->dX, e->hX, (size_t)Be * sizeof(int), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(e->dY, e->hY, (size_t)Be * sizeof(int), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(e->dSlot, e->hSlot, (size_t)Be * sizeof(int), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(e->dF, e->hF, (size_t)Be, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(e->dM, e->hM, sizeof(int), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(e->dSti, e->hSti, sizeof(int), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(e->dG, e->hG, sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+  eval_forward(h, e, 0);
+  k_topk_score<<<dim3(lblocks, parts), EV_THREADS, topk_score_smem_bytes(cap), st>>>(e->slot, n_cand > 0 ? e->dTkCand : nullptr, n_comp, k, cap,
+                                                                                     e->dTkK, e->dTkI, e->dTkMZ);
+  k_topk_merge<<<batch, TK_MERGE_THREADS, 0, st>>>(e->slot, parts, k, e->dTkK, e->dTkI, e->dTkMZ, e->dTkItems, e->dTkScores);
+  h->launches += 2;
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(items_out, e->dTkItems, n_out * sizeof(int), cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(scores_out, e->dTkScores, n_out * sizeof(float), cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
   return G4R_OK;
 }

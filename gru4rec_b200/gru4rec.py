@@ -528,6 +528,43 @@ class GRU4Rec:
             return pd.DataFrame(data=preds, index=predict_for_item_ids)
         return pd.DataFrame(data=preds, index=self.itemidmap.index)
 
+    def recommend_next_batch(self, session_ids, input_item_ids, k=20, predict_for_item_ids=None, batch=100):
+        '''
+        The k best next items of every event of the batch, selected on the device: the scores are those predict_next_batch
+        returns for the same call, but the items x batch matrix is never built or copied.  The session bookkeeping is the same
+        as predict_next_batch's (hidden state kept per batch coordinate while the session id stays the same), so calls of the
+        two methods can be interleaved on one model.
+        predict_for_item_ids: optional list of distinct item ids the recommendations are drawn from; for softmax / softmax_logit
+        the scores are normalised over this list, as predict_next_batch(..., predict_for_item_ids) does.
+        Returns (item_ids, scores): original item ids [events x k] and float32 scores [events x k]; row b answers event b,
+        sorted by score descending, ties broken by the lower item index.
+        '''
+        if self.error_during_train: raise Exception
+        if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)):
+            raise ValueError('k must be an integer, got %r' % (k,))
+        cand = None
+        if predict_for_item_ids is not None:
+            if pd.Index(predict_for_item_ids).has_duplicates:
+                raise ValueError('predict_for_item_ids contains duplicates')
+            cand = self.itemidmap[predict_for_item_ids].values
+        n_cand = self.n_items if cand is None else len(cand)
+        if not 1 <= k <= min(256, n_cand):
+            raise ValueError('k must be in 1 .. min(256, number of candidate items) = %d, got %d' % (min(256, n_cand), k))
+        in_idxs = self.itemidmap[input_item_ids].values
+        eng = self._ensure_engine(batch)
+        # session bookkeeping of predict_next_batch
+        if getattr(self, 'predict', None) is None or self.predict_batch != batch:
+            self.predict_batch = batch
+            eng.reset_eval_hidden()
+            self.current_session = np.ones(batch) * -1
+            self.predict = True
+        session_ids = np.asarray(session_ids)
+        reset = (session_ids != self.current_session)
+        if reset.any():
+            self.current_session = session_ids.copy()
+        idx, scores = eng.predict_topk(in_idxs, int(k), reset.astype(np.uint8), cand)
+        return self.itemidmap.index.to_numpy()[idx], scores
+
     # ---- persistence (gru4rec.py:742-781): pickle of the object with NumPy parameters ----
     def __getstate__(self):
         st = dict(self.__dict__)

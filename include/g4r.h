@@ -203,6 +203,13 @@ int g4r_set_eval_items(g4r_handle* h, const int64_t* items, int64_t n);
 /* predict_next_batch's device call: scores of all items for `batch` lanes; reset_mask zeroes lanes first
  * (gru4rec.py:712-717).  out: [batch x n_items] row-major. */
 int g4r_predict(g4r_handle* h, const int32_t* X, int32_t batch, const uint8_t* reset_mask, float* out);
+/* Top-k of the scores g4r_predict would return for the same call, without materialising them.  Advances the scoring-path
+ * hidden state exactly like g4r_predict (one event per lane; reset_mask as there).  cand/n_cand: optional candidate item
+ * indices (NULL/0 = whole catalogue; duplicates -> G4R_ERR_INVALID).  Out: items_out / scores_out [batch x k], each row
+ * sorted by score descending, ties by item index ascending; softmax-family scores normalised over the candidates.
+ * k must be in 1 .. min(256, number of candidates).  Out-of-range X or candidate index -> G4R_ERR_INDEX. */
+int g4r_predict_topk(g4r_handle* h, const int32_t* X, int32_t batch, const uint8_t* reset_mask,
+                     const int64_t* cand, int64_t n_cand, int32_t k, int32_t* items_out, float* scores_out);
 /* Zero the scoring-path hidden state (gru4rec.py:696-697). */
 int g4r_reset_eval_hidden(g4r_handle* h);
 

@@ -80,6 +80,7 @@ struct FastSmem {
   int sIt[2][FK_CT], sPos[2][FK_CT], sTc[2][FK_B], sYit[2][FK_B], sCb[2][2];
   int sFlag[4];
   alignas(8) unsigned long long mbar;
+  unsigned long long sTs[2];        // %globaltimer around F1's wait for the helper CTAs (stamped runs only)
   // GRU role: thin-slab phases (every GRU CTA owns a few output columns / rows and stages the full 32-lane operand)
   alignas(16) float gA[FK_B * 388];             // staged [32 x <=384] operand (H, Hold*r, da_h, dvec)
   alignas(16) float gW[8 * FK_LDS + FK_NW * FK_B * 5 + 16 * FK_B];      // this CTA's weight slab (<= 8 columns/rows of length <= 128) + reduction scratch
@@ -108,7 +109,8 @@ __device__ __forceinline__ void fk_load_idx(const ModelDev& md, SM& sm, int s, i
   if (tid == 64) { sm.sCb[buf][0] = cb; sm.sCb[buf][1] = ce; }
 }
 
-// issue the TMA prefetch of step s (rows are final once the previous step's updates are complete)
+// issue the TMA prefetch of step s (rows are final once the previous step's updates are complete; k_fast_t updates a
+// chunk's rows after arriving at the last column barrier, so it acquires FastSync::rows before calling this)
 template <class SM>
 __device__ __forceinline__ void fk_prefetch_rows(const ModelDev& md, SM& sm, int s, int n_steps, int buf, bool pw) {
   if (s >= n_steps) return;
@@ -166,10 +168,28 @@ __device__ __forceinline__ void fk_prefetch_rows(const ModelDev& md, SM& sm, int
   }
 }
 
+// the TMA prefetch of step s + 1 once every CTA's chunk-row update of step s is complete
+template <class SM>
+__device__ __forceinline__ void fk_wait_rows_prefetch(const ModelDev& md, SM& sm, FastSync* fs, int s, int n_steps, int buf, bool pw, int ncta) {
+  if (s + 1 >= n_steps) return;
+  if (threadIdx.x == 0) wait_ge(&fs->rows, (unsigned int)(s + 1) * (unsigned int)ncta);
+  __syncthreads();
+  fk_prefetch_rows(md, sm, s + 1, n_steps, buf ^ 1, pw);
+}
 __device__ __forceinline__ void fk_group_barrier(FastSync* fs, unsigned int& gepoch) {
   __syncthreads();
   gepoch += 1;
   if (threadIdx.x == 0) { red_release_add(&fs->grp, 1u); wait_ge(&fs->grp, gepoch * FK_G); }
+  __syncthreads();
+}
+// the same barrier split in two, so that work which needs no other CTA runs while the group arrives
+__device__ __forceinline__ void fk_group_arrive(FastSync* fs, unsigned int& gepoch) {
+  __syncthreads();
+  gepoch += 1;
+  if (threadIdx.x == 0) red_release_add(&fs->grp, 1u);
+}
+__device__ __forceinline__ void fk_group_wait(FastSync* fs, unsigned int gepoch) {
+  if (threadIdx.x == 0) wait_ge(&fs->grp, gepoch * FK_G);
   __syncthreads();
 }
 
@@ -222,24 +242,34 @@ __device__ __forceinline__ float fk_slab_reduce(const float (&acc)[W], float* re
 constexpr int FK_W1 = 5;    // rz columns per CTA   (ceil(2*128 / 48) = 6 would also fit; 2L <= 240 with 48 CTAs)
 constexpr int FK_W2 = 3;    // h / dHr columns per CTA (L <= 144)
 
+// stage H rows of the lanes (fk_stage_lanes done; zero for out-of-range lanes) for F1
+__device__ __forceinline__ void fk_f1_stage_h(const LayerDev& ly, FastSmem& sm) {
+  const int ldL = ly.ldL;
+  stage_rows4(sm.gA, FK_LDS, FK_B, ldL / 4, [&](int rr) -> const float* { const int sl = sm.gIdx[rr]; return sl >= 0 ? ly.H + (size_t)sl * ldL : nullptr; });
+}
 // F1: rz = sigmoid(Wx0[X][L:3L] + Bh[L:3L] + H @ Wrz) for this CTA's FK_W1 columns; CTA 0 also writes Hold
 // inrows != nullptr (row-sharded multi-GPU): the gathered input rows Wx0[X] of the step sit in a local [B x ld3] buffer
-__device__ void fk_f1(const ModelDev& md, FastSmem& sm, int s, int cta, const unsigned int* wait_ctr, unsigned int wait_target, const float* inrows = nullptr) {
+// staged: the lanes (fk_stage_lanes), the H rows (fk_f1_stage_h) and the transposed weight slab gW[j][k] = Wrz[k][c0 + j]
+// (zero outside j < W, k < L) are already in shared memory, otherwise they are staged from global memory here
+// stamp: the %globaltimer around the wait for the helper CTAs goes to sm.sTs (equal stamps when no wait was needed)
+__device__ void fk_f1(const ModelDev& md, FastSmem& sm, int s, int cta, const unsigned int* wait_ctr, unsigned int wait_target, const float* inrows = nullptr,
+                      bool staged = false, bool stamp = false) {
   const LayerDev& ly = md.layer[0];
   const int M = md.wM[s], L = ly.L, ldL = ly.ldL, tid = threadIdx.x;
   const int c0 = cta * FK_W1;
   if (c0 >= 2 * L) return;
   const int W = min(FK_W1, 2 * L - c0);
-  fk_stage_lanes(md, sm, s, M);
-  // if the helper CTAs' input-row updates are already complete (the usual case), the epilogue operand is fetched before the
-  // product instead of after it
+  if (!staged) fk_stage_lanes(md, sm, s, M);
+  // if the helper CTAs' input-row updates are already complete, the epilogue operand is fetched before the product instead
+  // of after it
   if (tid == 0) sm.sFlag[3] = (!wait_ctr || ld_acquire_u32(wait_ctr) >= wait_target) ? 1 : 0;
   const int kw = ldL / 4;
-  // stage H rows (zero for out-of-range lanes) and the transposed weight slab Wt[j][k] = Wrz[k][c0 + j]
-  stage_rows4(sm.gA, FK_LDS, FK_B, kw, [&](int rr) -> const float* { const int sl = sm.gIdx[rr]; return sl >= 0 ? ly.H + (size_t)sl * ldL : nullptr; });
-  for (int i = tid; i < FK_W1 * FK_LDS; i += FK_THREADS) {
-    const int j = i / FK_LDS, k = i % FK_LDS;
-    sm.gW[i] = (j < W && k < L) ? ly.Wrz[(size_t)k * ly.ld2 + c0 + j] : 0.f;
+  if (!staged) {
+    fk_f1_stage_h(ly, sm);
+    for (int i = tid; i < FK_W1 * FK_LDS; i += FK_THREADS) {
+      const int j = i / FK_LDS, k = i % FK_LDS;
+      sm.gW[i] = (j < W && k < L) ? ly.Wrz[(size_t)k * ly.ld2 + c0 + j] : 0.f;
+    }
   }
   const int b = tid & 31, jsel = tid >> 5;
   __syncthreads();
@@ -251,11 +281,13 @@ __device__ void fk_f1(const ModelDev& md, FastSmem& sm, int s, int cta, const un
   const float v = fk_slab_reduce<FK_W1>(acc, sm.gW + 8 * FK_LDS, jsel);
   // otherwise the gathered input rows are still in flight on the helper CTAs (previous step's update): wait now, after
   // the H @ Wrz part, then fetch the epilogue operands (gathered row element + bias)
+  if (stamp && tid == 0) { unsigned long long t_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_)); sm.sTs[0] = t_; }
   if (!early) {
     if (tid == 0) wait_ge(wait_ctr, wait_target);
     __syncthreads();
     if (jsel < W && b < M) pre = (inrows ? inrows[(size_t)b * ly.ld3 + L + c0 + jsel] : ly.Wx[(size_t)sm.gIdx[FK_B + b] * ly.ld3 + L + c0 + jsel]) + ly.Bh[L + c0 + jsel];
   }
+  if (stamp && tid == 0) { unsigned long long t_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_)); sm.sTs[1] = t_; }
   if (jsel < W && b < M) {
     const int c = c0 + jsel;
     const float g = sigmoidf_(v + pre);
@@ -269,13 +301,16 @@ __device__ void fk_f1(const ModelDev& md, FastSmem& sm, int s, int cta, const un
   }
 }
 // F2: h~ = act(Wx0[X][0:L] + Bh[0:L] + (H*r) @ Wh), h, dropout, H_new for this CTA's FK_W2 columns
-__device__ void fk_f2(const ModelDev& md, FastSmem& sm, int s, int cta, const float* inrows = nullptr) {
+// staged: the lanes of step s (fk_stage_lanes) and the transposed slab Wt[j][k] = Wh[k][c0 + j] (zero outside j < W, k < L)
+// are already in shared memory, the slab at rows FK_W1.. of gW (after F1's Wrz rows); otherwise both are staged here, the slab
+// from global memory to rows 0..
+__device__ void fk_f2(const ModelDev& md, FastSmem& sm, int s, int cta, const float* inrows = nullptr, bool staged = false) {
   const LayerDev& ly = md.layer[0];
   const int M = md.wM[s], L = ly.L, ldL = ly.ldL, tid = threadIdx.x;
   const int c0 = cta * FK_W2;
   if (c0 >= L) return;
   const int W = min(FK_W2, L - c0);
-  fk_stage_lanes(md, sm, s, M);
+  if (!staged) fk_stage_lanes(md, sm, s, M);
   const int kw = ldL / 4;
   // stage H*r
   for (int i0 = 0; i0 < FK_B * kw; i0 += 2 * FK_THREADS) {
@@ -295,9 +330,11 @@ __device__ void fk_f2(const ModelDev& md, FastSmem& sm, int s, int cta, const fl
       if (i < FK_B * kw) st4(sm.gA + (i / kw) * FK_LDS + (i % kw) * 4, make_float4(hv[u].x * rv[u].x, hv[u].y * rv[u].y, hv[u].z * rv[u].z, hv[u].w * rv[u].w));
     }
   }
-  for (int i = tid; i < FK_W2 * FK_LDS; i += FK_THREADS) {
-    const int j = i / FK_LDS, k = i % FK_LDS;
-    sm.gW[i] = (j < W && k < L) ? ly.Wh[(size_t)k * ldL + c0 + j] : 0.f;
+  if (!staged) {
+    for (int i = tid; i < FK_W2 * FK_LDS; i += FK_THREADS) {
+      const int j = i / FK_LDS, k = i % FK_LDS;
+      sm.gW[i] = (j < W && k < L) ? ly.Wh[(size_t)k * ldL + c0 + j] : 0.f;
+    }
   }
   const int b = tid & 31, jsel = tid >> 5;
   float pre = 0.f, z = 0.f, ho = 0.f;
@@ -309,7 +346,7 @@ __device__ void fk_f2(const ModelDev& md, FastSmem& sm, int s, int cta, const fl
   }
   __syncthreads();
   float acc[FK_W2];
-  fk_slab_dot<FK_W2>(acc, sm.gA, FK_LDS, sm.gW, L);
+  fk_slab_dot<FK_W2>(acc, sm.gA, FK_LDS, sm.gW + (staged ? FK_W1 * FK_LDS : 0), L);
   const float v0 = fk_slab_reduce<FK_W2>(acc, sm.gW + 8 * FK_LDS, jsel);
   if (jsel < W && b < M) {
     const int c = c0 + jsel;
@@ -343,81 +380,131 @@ __device__ void fk_b2(const ModelDev& md, FastSmem& sm, int s, int cta) {
   const float v = fk_slab_reduce<FK_W2>(acc, sm.gW + 8 * FK_LDS, jsel);
   if (jsel < W && b < M) ly.dvec[(size_t)b * ly.ld3 + L + c0 + jsel] = v * ho * r * (1.f - r);
 }
-// D: dense gradients of this CTA's row slab of Wh / Wrz (and a slice of Bh) fused with their Adagrad(+momentum) update
-__device__ void fk_dense(const ModelDev& md, FastSmem& sm, int s, int cta) {
-  const LayerDev& ly = md.layer[0];
-  const int M = md.wM[s], L = ly.L, ldL = ly.ldL, ld3 = ly.ld3, tid = threadIdx.x;
-  const int R = (L + FK_G - 1) / FK_G;            // rows of Wh / Wrz per CTA
-  const int k0 = cta * R;
-  const int nr = max(0, min(R, L - k0));
-  const int CB = (3 * L + FK_G - 1) / FK_G;       // Bh entries per CTA
-  const int cb0 = cta * CB, ncb = max(0, min(CB, 3 * L - cb0));
-  if (nr == 0 && ncb == 0) return;
-  float* sHo = sm.gW;                  // [R][32]
-  float* sHr = sm.gW + 8 * FK_B;       // [R][32]
-  // outputs: nr x L (Wh), nr x 2L (Wrz), ncb (Bh).  Each thread owns U outputs at a time: their parameter / Adagrad /
-  // momentum values are loaded first, the U batch reductions (<= 32 lanes) run interleaved, then the updates are stored.
-  const int nWh = nr * L, nWrz = nr * 2 * L, total = nWh + nWrz + ncb;
-  constexpr int U = 2;
-  const bool ada = md.adapt == G4R_ADAPT_ADAGRAD, mom = md.mom > 0.f;
-  float* p[U]; float* pa[U]; float* pv[U]; const float* av[U]; const float* bv[U]; bool ok[U]; bool bias[U];
-  float p0[U], a0[U], v0[U], g[U];
-  auto load_ops = [&](int o0) {
-#pragma unroll
-    for (int u = 0; u < U; u++) {
-      const int o = o0 + u * FK_THREADS + tid;
-      ok[u] = o < total; bias[u] = false; p[u] = nullptr; pa[u] = nullptr; pv[u] = nullptr; av[u] = sHo; bv[u] = sm.gA;
-      if (ok[u]) {
-        if (o < nWh) {
-          const int rr = o / L, c = o % L;
-          const size_t off = (size_t)(k0 + rr) * ldL + c;
-          p[u] = ly.Wh + off; pa[u] = ly.Wh_acc ? ly.Wh_acc + off : nullptr; pv[u] = ly.Wh_vel ? ly.Wh_vel + off : nullptr;
-          av[u] = sHr + rr * FK_B; bv[u] = sm.gA + c;
-        } else if (o < nWh + nWrz) {
-          const int q = o - nWh, rr = q / (2 * L), c = q % (2 * L);
-          const size_t off = (size_t)(k0 + rr) * ly.ld2 + c;
-          p[u] = ly.Wrz + off; pa[u] = ly.Wrz_acc ? ly.Wrz_acc + off : nullptr; pv[u] = ly.Wrz_vel ? ly.Wrz_vel + off : nullptr;
-          av[u] = sHo + rr * FK_B; bv[u] = sm.gA + L + c;
-        } else {
-          const int c = cb0 + (o - nWh - nWrz);
-          p[u] = ly.Bh + c; pa[u] = ly.Bh_acc ? ly.Bh_acc + c : nullptr; pv[u] = ly.Bh_vel ? ly.Bh_vel + c : nullptr;
-          bias[u] = true; bv[u] = sm.gA + c;
-        }
-      }
-      p0[u] = ok[u] ? *p[u] : 0.f;
-      a0[u] = (ok[u] && ada && pa[u]) ? *pa[u] : 0.f;
-      v0[u] = (ok[u] && mom && pv[u]) ? *pv[u] : 0.f;
-      g[u] = 0.f;
-    }
-  };
-  // this CTA's rows of Wh / Wrz / Bh are written by nobody else: the operands of the first pass are fetched before the
-  // dvec rows are staged, so the two global round trips overlap
-  load_ops(0);
-  __syncthreads();
-  // stage dvec [32 x 3L] and the (Hold, Hold*r) columns of this slab
-  // 32 x 75 quads at L = 100: five loads in flight per thread cover the whole block in one round trip
-  stage_rows_n<5>(sm.gA, 388, FK_B, ld3 / 4, [&](int rr) -> const float* { return rr < M ? ly.dvec + (size_t)rr * ld3 : nullptr; });
-  for (int i = tid; i < nr * FK_B; i += FK_THREADS) {
-    const int rr = i / FK_B, b = i % FK_B;
-    float ho = 0.f, r = 0.f;
-    if (b < M) { ho = ly.Hold[(size_t)b * ldL + k0 + rr]; r = ly.r[(size_t)b * ldL + k0 + rr]; }
-    sHo[i] = ho; sHr[i] = ho * r;
+// D: dense Adagrad(+momentum) of Wh / Wrz / Bh, owned by the forward column owners.  GRU CTA `cta` updates exactly the
+// weights it multiplies with in F1 / F2 of the next step, so the updated slab feeds those products from shared memory:
+//   e = j L + k            (j < FK_W1)  Wrz[k][c0 + j], c0 = FK_W1 cta    grad sum_b Hold[b][k] dvec[b][L + c0 + j]
+//   e = (FK_W1 + j) L + k  (j < FK_W2)  Wh[k][c2 + j],  c2 = FK_W2 cta    grad sum_b (Hold r)[b][k] dvec[b][c2 + j]
+//   e = FK_WD L + j                     Bh[L + c0 + j] (j < FK_W1), Bh[c2 + j - FK_W1]     grad sum_b of the same column
+// Only this CTA reads or writes these values, except Wh, which B2 reads by rows before the group barrier that follows it.
+// Per element the arithmetic is the generic dense update's: the lanes summed in order with fmaf (the bias: plain sums), then
+// adagrad_scale and dense_step.  The Wr columns (and Bh_r) need da_r from every CTA's B2 and run after that barrier
+// (phase 1); everything else runs while the CTA waits for it (phase 0).
+constexpr int FK_WD = FK_W1 + FK_W2;                 // slab rows: F1 columns, then F2 columns
+constexpr int FK_DNE = FK_WD * 120 + FK_WD;          // owned elements per GRU CTA at L <= 120
+static_assert(3 * FK_DNE <= FK_NW * FK_B * 8, "owned parameter / Adagrad / momentum values fit sPart");
+static_assert(2 * FK_B * FK_LDS <= FK_B * 388, "Hold * r fits behind the staged H rows in gA");
+static_assert(FK_WD * FK_B <= FK_CT * FK_B, "owned dvec columns fit sG");
+
+// owned element e: parameter / Adagrad / momentum pointers, slab row j, weight row k (-1: bias); false if e is past the layer
+__device__ __forceinline__ bool fk_own(const LayerDev& ly, int cta, int e, float*& p, float*& pa, float*& pv, int& j, int& k) {
+  const int L = ly.L, c0 = cta * FK_W1, c2 = cta * FK_W2;
+  size_t off;
+  if (e < FK_WD * L) { j = e / L; k = e % L; }
+  else { j = e - FK_WD * L; k = -1; if (j >= FK_WD) return false; }
+  if (j < FK_W1 ? c0 + j >= 2 * L : c2 + j - FK_W1 >= L) return false;
+  if (k < 0) {
+    off = j < FK_W1 ? (size_t)(L + c0 + j) : (size_t)(c2 + j - FK_W1);
+    p = ly.Bh + off; pa = ly.Bh_acc ? ly.Bh_acc + off : nullptr; pv = ly.Bh_vel ? ly.Bh_vel + off : nullptr;
+  } else if (j < FK_W1) {
+    off = (size_t)k * ly.ld2 + c0 + j;
+    p = ly.Wrz + off; pa = ly.Wrz_acc ? ly.Wrz_acc + off : nullptr; pv = ly.Wrz_vel ? ly.Wrz_vel + off : nullptr;
+  } else {
+    off = (size_t)k * ly.ldL + c2 + j - FK_W1;
+    p = ly.Wh + off; pa = ly.Wh_acc ? ly.Wh_acc + off : nullptr; pv = ly.Wh_vel ? ly.Wh_vel + off : nullptr;
   }
-  __syncthreads();
-  for (int o0 = 0; o0 < total; o0 += U * FK_THREADS) {
-    if (o0 > 0) load_ops(o0);
-    for (int b = 0; b < M; b++) {
+  return true;
+}
+// phase of slab row j: 1 for the Wr columns (their gradient needs da_r), 0 otherwise
+__device__ __forceinline__ int fk_own_phase(int L, int cta, int j) { return (j < FK_W1 && cta * FK_W1 + j < L) ? 1 : 0; }
+
+// While the CTA waits for b1_done: Hold(s) and Hold * r(s) into shared memory (F1 of step s + 1 overwrites both in global
+// memory after the B2 group barrier), and the owned parameter / Adagrad / momentum values (final: no other CTA writes them).
+// All loads are issued before the first store, so the whole staging costs one round trip.
+__device__ void fk_dense_stage(const ModelDev& md, FastSmem& sm, int s, int cta) {
+  const LayerDev& ly = md.layer[0];
+  const int M = md.wM[s], L = ly.L, ldL = ly.ldL, kw = ldL / 4, tid = threadIdx.x;
+  if (cta * FK_W1 >= 2 * L) return;                 // no F1 columns (and so no F2 columns either)
+  const bool ada = md.adapt == G4R_ADAPT_ADAGRAD, mom = md.mom > 0.f;
+  constexpr int NU = 2;                             // M * kw <= 32 * 32 quads and FK_DNE elements: two per thread
+  static_assert(NU * FK_THREADS >= FK_B * 32 && NU * FK_THREADS >= FK_DNE, "fk_dense_stage covers one pass");
+  float4 hv[NU], rv[NU];
+  float p0[NU], a0[NU], v0[NU];
 #pragma unroll
-      for (int u = 0; u < U; u++) g[u] = bias[u] ? g[u] + bv[u][b * 388] : fmaf(av[u][b], bv[u][b * 388], g[u]);
+  for (int u = 0; u < NU; u++) {
+    const int i = u * FK_THREADS + tid;
+    hv[u] = make_float4(0.f, 0.f, 0.f, 0.f); rv[u] = hv[u];
+    if (i < M * kw) { const size_t o = (size_t)(i / kw) * ldL + (i % kw) * 4; hv[u] = ld4(ly.Hold + o); rv[u] = ld4(ly.r + o); }
+    float *p, *pa, *pv; int j, k;
+    p0[u] = 0.f; a0[u] = 0.f; v0[u] = 0.f;
+    if (fk_own(ly, cta, i, p, pa, pv, j, k)) {
+      p0[u] = *p;
+      if (ada && pa) a0[u] = *pa;
+      if (mom && pv) v0[u] = *pv;
     }
+  }
+  float* sHr = sm.gA + FK_B * FK_LDS;
 #pragma unroll
-    for (int u = 0; u < U; u++) {
-      if (!ok[u]) continue;
-      float gs = g[u];
-      if (ada) gs = adagrad_scale(g[u], a0[u], *pa[u]);
-      float v = v0[u];
-      *p[u] = dense_step(md, gs, p0[u], v, mom);
-      if (mom) *pv[u] = v;
+  for (int u = 0; u < NU; u++) {
+    const int i = u * FK_THREADS + tid;
+    if (i < M * kw) {
+      const int o = (i / kw) * FK_LDS + (i % kw) * 4;
+      st4(sm.sD + o, hv[u]);
+      st4(sHr + o, make_float4(hv[u].x * rv[u].x, hv[u].y * rv[u].y, hv[u].z * rv[u].z, hv[u].w * rv[u].w));
+    }
+    if (i < FK_DNE) { sm.sPart[i] = p0[u]; sm.sPart[FK_DNE + i] = a0[u]; sm.sPart[2 * FK_DNE + i] = v0[u]; }
+  }
+}
+// this thread's element of the owned dvec columns of phase ph (tid = j * FK_B + b), for fk_dense_put_dcol
+__device__ __forceinline__ float fk_dense_dcol(const LayerDev& ly, int M, int cta, int ph) {
+  const int j = threadIdx.x / FK_B, b = threadIdx.x % FK_B, L = ly.L, c0 = cta * FK_W1, c2 = cta * FK_W2;
+  if (j >= FK_WD || b >= M || fk_own_phase(L, cta, j) != ph) return 0.f;
+  if (j < FK_W1 ? c0 + j >= 2 * L : c2 + j - FK_W1 >= L) return 0.f;
+  return ly.dvec[(size_t)b * ly.ld3 + (j < FK_W1 ? L + c0 + j : c2 + j - FK_W1)];
+}
+__device__ __forceinline__ void fk_dense_put_dcol(FastSmem& sm, const LayerDev& ly, int cta, int ph, float v) {
+  const int j = threadIdx.x / FK_B;
+  if (j < FK_WD && fk_own_phase(ly.L, cta, j) == ph) sm.sG[threadIdx.x] = v;
+}
+// gradient and update of the owned elements of phase ph (fk_dense_stage and fk_dense_put_dcol of the phase done).  The new
+// weights go to the slab rows gW[j][k] (zero elsewhere) that F1 / F2 multiply with, and to global memory; the Wh
+// parameters only in phase 1, once every CTA has passed B2.
+__device__ void fk_dense_update(const ModelDev& md, FastSmem& sm, int s, int cta, int ph) {
+  const LayerDev& ly = md.layer[0];
+  const int M = md.wM[s], L = ly.L, tid = threadIdx.x;
+  if (cta * FK_W1 >= 2 * L) return;
+  const bool ada = md.adapt == G4R_ADAPT_ADAGRAD, mom = md.mom > 0.f;
+  const float* sHr = sm.gA + FK_B * FK_LDS;
+  if (ph == 0) {
+    for (int i = tid; i < FK_WD * FK_LDS; i += FK_THREADS) {
+      const int j = i / FK_LDS, k = i % FK_LDS;
+      float *p, *pa, *pv; int jj, kk;
+      if (k >= L || !fk_own(ly, cta, j * L, p, pa, pv, jj, kk)) sm.gW[i] = 0.f;
+    }
+  }
+  for (int e = tid; e < FK_WD * L + FK_WD; e += FK_THREADS) {
+    float *p, *pa, *pv; int j, k;
+    if (!fk_own(ly, cta, e, p, pa, pv, j, k) || fk_own_phase(L, cta, j) != ph) continue;
+    const float* dc = sm.sG + j * FK_B;
+    float g = 0.f;
+    if (k >= 0) {
+      const float* a = (j < FK_W1 ? sm.sD : sHr) + k;
+      for (int b = 0; b < M; b++) g = fmaf(a[b * FK_LDS], dc[b], g);
+    } else {
+      for (int b = 0; b < M; b++) g = g + dc[b];
+    }
+    float gs = g;
+    if (ada) gs = adagrad_scale(g, sm.sPart[FK_DNE + e], *pa);
+    float v = sm.sPart[2 * FK_DNE + e];
+    const float pn = dense_step(md, gs, sm.sPart[e], v, mom);
+    if (mom) *pv = v;
+    if (k >= 0) sm.gW[j * FK_LDS + k] = pn;
+    if (k < 0 || j < FK_W1) *p = pn;
+  }
+  if (ph == 1) {
+    const int c2 = cta * FK_W2, W2 = max(0, min(FK_W2, L - c2));
+    for (int i = tid; i < W2 * L; i += FK_THREADS) {
+      const int k = i / W2, j = i % W2;
+      ly.Wh[(size_t)k * ly.ldL + c2 + j] = sm.gW[(FK_W1 + j) * FK_LDS + k];
     }
   }
 }
@@ -569,6 +656,8 @@ __global__ void __launch_bounds__(FK_THREADS, 1) k_fast_t(int slot, int n_steps,
 #define FK_STAMP_OK(s_) true
 #endif
 #define FK_STAMP(k) do { if (tstamp && cta == 0 && tid == 0 && FK_STAMP_OK(s)) { unsigned long long t_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_)); tstamp[(size_t)s * 16 + (k)] = t_; } } while (0)
+// fine stamps of the column phases; in step_mode 2 the GRU role reuses their slots (1, 4, 9, 10, 11, 12)
+#define FK_STAMP_CL(k) do { if (CL) FK_STAMP(k); } while (0)
   if (tid == 0) { mbar_init(bar, 1); asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
   fk_load_idx(md, sm, 0, n_steps, chunk, 0);
   __syncthreads();
@@ -610,7 +699,7 @@ __global__ void __launch_bounds__(FK_THREADS, 1) k_fast_t(int slot, int n_steps,
     stage_rows4(sm.sY, FK_LDS, FK_B, kw, [&](int rr) -> const float* { return rr < M ? ly.y + (size_t)rr * ldL : nullptr; });
     mbar_wait(bar, (unsigned int)(s & 1));      // prefetched rows of this step have landed
     __syncthreads();
-    FK_STAMP(1);
+    FK_STAMP_CL(1);
     const int cb = sm.sCb[buf][0], ce = sm.sCb[buf][1];
     const int nj = ce - cb;
     // ---- scores + partial statistics ----
@@ -642,7 +731,7 @@ __global__ void __launch_bounds__(FK_THREADS, 1) k_fast_t(int slot, int n_steps,
           }
         }
       }
-      FK_STAMP(9);
+      FK_STAMP_CL(9);
 #pragma unroll
       for (int q = 0; q < FK_Q; q++) {
         const int jj = warp + q * FK_NW;
@@ -696,7 +785,7 @@ __global__ void __launch_bounds__(FK_THREADS, 1) k_fast_t(int slot, int n_steps,
     }
     // ---- barrier B2, then lane b's statistics are combined by CTA b (all lanes in parallel, fixed merge order) ----
     __syncthreads();
-    FK_STAMP(10);
+    FK_STAMP_CL(10);
     bar_epoch += 1;
     if (tid == 0) { red_release_add(&fs->bar, 1u); wait_ge(&fs->bar, bar_epoch * (unsigned int)ncta); }
     __syncthreads();
@@ -762,7 +851,7 @@ __global__ void __launch_bounds__(FK_THREADS, 1) k_fast_t(int slot, int n_steps,
       md.cost[s] = c;
       if (c != c) atomicExch(md.nanflag, 1);
     }
-    FK_STAMP(11);
+    FK_STAMP_CL(11);
     for (int i = tid; i < FK_CT * FK_B; i += FK_THREADS) {
       const int jj = i / FK_B, b = i % FK_B;
       sm.sG[i] = (jj < nj && b < M) ? loss_grad_elem(md, sm.sRS + (size_t)b * 8, sm.sO[i], sm.sTc[buf][b] == cb + jj, M, N) : 0.f;
@@ -773,7 +862,7 @@ __global__ void __launch_bounds__(FK_THREADS, 1) k_fast_t(int slot, int n_steps,
       a = warp_sum(a);
       if (lane == 0) sm.sDby[jj] = a;
     }
-    FK_STAMP(12);
+    FK_STAMP_CL(12);
     float* part = md.part + (size_t)(has_chunk ? chunk : 0) * md.B * ldL;
     if (has_chunk) {
       // dSy[j][quad] = sum_b g[b][j] y[b][quad]: one thread per (column, 16-byte feature quad), all nj*kw pairs in parallel
@@ -799,10 +888,15 @@ __global__ void __launch_bounds__(FK_THREADS, 1) k_fast_t(int slot, int n_steps,
         st4(part + (size_t)bb * ldL + q4 * 4, a);
       }
     }
+    if (has_chunk && nj == 0) for (int i = tid; i < M * ldL; i += FK_THREADS) part[i] = 0.f;
+    // ---- barrier B3: partial dL/dh complete.  Arrive, update the chunk's rows while the others arrive, then wait ----
     __syncthreads();
     FK_STAMP(13);
-    // sparse update from shared memory (rows prefetched before the step): one warp per duplicate group.  Written out
-    // rather than with SparseUpd4 / SparseUpd, which cost this kernel a 16-byte register spill; same arithmetic.
+    bar_epoch += 1;
+    if (tid == 0) red_release_add(&fs->bar, 1u);
+    // sparse update from shared memory (rows prefetched before the step): one warp per duplicate group.  Nothing before the
+    // next step's prefetch reads these rows, which waits for fs->rows.  Written out rather than with SparseUpd4 / SparseUpd,
+    // which cost this kernel a 16-byte register spill; same arithmetic.
     for (int j = warp; j < nj; j += FK_THREADS / 32) {
       const int item = sm.sIt[buf][j];
       if (j > 0 && sm.sIt[buf][j - 1] == item) continue;
@@ -850,12 +944,10 @@ __global__ void __launch_bounds__(FK_THREADS, 1) k_fast_t(int slot, int n_steps,
         if (mom) md.By_vel[item] = vl;
       }
     }
-    if (has_chunk && nj == 0) for (int i = tid; i < M * ldL; i += FK_THREADS) part[i] = 0.f;
-    // ---- barrier B3: all updates and partial dL/dh complete ----
     __syncthreads();
+    if (tid == 0) red_release_add(&fs->rows, 1u);
     FK_STAMP(14);
-    bar_epoch += 1;
-    if (tid == 0) { red_release_add(&fs->bar, 1u); wait_ge(&fs->bar, bar_epoch * (unsigned int)ncta); }
+    if (tid == 0) wait_ge(&fs->bar, bar_epoch * (unsigned int)ncta);
     __syncthreads();
     FK_STAMP(3);
     // ---- b1 on every CTA, then prefetch the next step's rows ----
@@ -863,8 +955,16 @@ __global__ void __launch_bounds__(FK_THREADS, 1) k_fast_t(int slot, int n_steps,
     __syncthreads();
     if (tid == 0) red_release_add(&fs->b1_done, 1u);
     FK_STAMP(15);
-    fk_prefetch_rows(md, sm, s + 1, n_steps, buf ^ 1, pw);
-    FK_STAMP(4);
+    // prefetch of the next step's rows, which any CTA may have updated inside its B3 window (the GRU CTAs of step_mode 2
+    // issue it inside the B2 group-barrier window instead)
+    if (CL || !gru) fk_wait_rows_prefetch(md, sm, fs, s, n_steps, buf, pw, ncta);
+    FK_STAMP_CL(4);
+    if constexpr (!CL) {
+      if (gru) {                                  // during the b1_done wait: operands of the dense update, lanes of the next step
+        fk_dense_stage(md, sm, s, cta);
+        if (s + 1 < n_steps) fk_stage_lanes(md, sm, s + 1, md.wM[s + 1]);
+      }
+    }
     // ---- GRU role: backward, dense update, forward of the next step ----
     if constexpr (CL) {
       if (gru) {
@@ -895,24 +995,43 @@ __global__ void __launch_bounds__(FK_THREADS, 1) k_fast_t(int slot, int n_steps,
     } else if (gru) {
       if (tid == 0) wait_ge(&fs->b1_done, (unsigned int)(s + 1) * (unsigned int)ncta);
       __syncthreads();
+      const float dc0 = fk_dense_dcol(ly, M, cta, 0);  // da_h / da_z columns of the owned slab: in flight during b2
       fk_b2(md, sm, s, cta);
-      fk_group_barrier(fs, gepoch);      // epoch 3*s + 2: all of dvec (da_r included) is complete -> the helper CTAs poll this counter
+      fk_group_arrive(fs, gepoch);       // epoch 2*s + 2: all of dvec (da_r included) is complete -> the helper CTAs poll this counter
       FK_STAMP(5);
-      fk_dense(md, sm, s, cta);
-      fk_group_barrier(fs, gepoch);
+      if (s + 1 < n_steps) {                     // the prefetch, inside the window: wait for every CTA's row update...
+        if (tid == 0) wait_ge(&fs->rows, (unsigned int)(s + 1) * (unsigned int)ncta);
+        __syncthreads();
+      }
+      FK_STAMP(4);
+      fk_prefetch_rows(md, sm, s + 1, n_steps, buf ^ 1, pw);   // ...then issue the copies
+      FK_STAMP(10);
+      fk_dense_put_dcol(sm, ly, cta, 0, dc0);
+      __syncthreads();
+      fk_dense_update(md, sm, s, cta, 0);
+      if (s + 1 < n_steps && cta * FK_W1 < 2 * L) fk_f1_stage_h(ly, sm);
+      FK_STAMP(1);
+      fk_group_wait(fs, gepoch);
+      FK_STAMP(9);
+      const float dc1 = fk_dense_dcol(ly, M, cta, 1);  // da_r columns
+      fk_dense_put_dcol(sm, ly, cta, 1, dc1);
+      __syncthreads();
+      fk_dense_update(md, sm, s, cta, 1);
+      __syncthreads();
       FK_STAMP(6);
       if (s + 1 < n_steps) {
-        fk_f1(md, sm, s + 1, cta, &fs->in_done, (unsigned int)(s + 1) * (unsigned int)in_ctas);   // waits for the helper CTAs' input-row updates
+        fk_f1(md, sm, s + 1, cta, &fs->in_done, (unsigned int)(s + 1) * (unsigned int)in_ctas, nullptr, true, tstamp && cta == 0);   // waits for the helper CTAs' input-row updates
         fk_group_barrier(fs, gepoch);
         FK_STAMP(7);
-        fk_f2(md, sm, s + 1, cta);
+        if (tstamp && cta == 0 && tid == 0 && FK_STAMP_OK(s)) { tstamp[(size_t)s * 16 + 11] = sm.sTs[0]; tstamp[(size_t)s * 16 + 12] = sm.sTs[1]; }
+        fk_f2(md, sm, s + 1, cta, nullptr, true);
         __syncthreads();
         if (tid == 0) red_release_add(&fs->h_ready, 1u);
       }
       FK_STAMP(8);
     } else if (cta < FK_G + in_ctas) {
-      // the GRU group's barrier after B2 is its (3 s + 2)-th group barrier (1 in the prologue, then B2 / dense / f1 per step)
-      if (tid == 0) wait_ge(&fs->grp, (unsigned int)(3 * s + 2) * FK_G);
+      // the GRU group's barrier after B2 is its (2 s + 2)-th group barrier (1 in the prologue, then B2 / f1 per step)
+      if (tid == 0) wait_ge(&fs->grp, (unsigned int)(2 * s + 2) * FK_G);
       __syncthreads();
       for (int b = cta - FK_G; b < B; b += in_ctas) { fk_sparse_in(md, sm, s, b); __syncthreads(); }
       __syncthreads();
@@ -921,4 +1040,5 @@ __global__ void __launch_bounds__(FK_THREADS, 1) k_fast_t(int slot, int n_steps,
   }
   if constexpr (CL) { if (gru) cf_store_resident(md, sm, cc); }
 #undef FK_STAMP
+#undef FK_STAMP_CL
 }

@@ -101,6 +101,7 @@ struct FastSync {                   // one counter per 128-byte line
   unsigned int b1_done;  unsigned int p3[31];
   unsigned int grp;      unsigned int p4[31];
   unsigned int in_done;  unsigned int p5[31];
+  unsigned int rows;     unsigned int p6[31];   // k_fast_t: chunk-row (Wy / By) updates of a step complete
 };
 struct GridBar { unsigned int count; unsigned int gen; unsigned int pad[30]; };   // grid barrier state (persistent mode)
 

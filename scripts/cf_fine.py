@@ -7,14 +7,15 @@ import numpy as np
 import bench
 from gru4rec_b200 import _lib
 import gru4rec as g4
-mk = dict(bench.WORKLOAD['model'])
+wl = bench.WORKLOADS['cfg2']                  # the headline workload of bench.py
+mk = dict(wl['model'])
 K = 1000
-cfg = _lib.make_config(bench.WORKLOAD['n_items'], mk, sample_store=bench.WORKLOAD['sample_store'], max_resident_steps=K + 8, step_mode=3)
+cfg = _lib.make_config(wl['n_items'], mk, sample_store=bench.SAMPLE_STORE, max_resident_steps=K + 8, step_mode=3)
 eng = _lib.Engine(cfg)
-gru = g4.GRU4Rec(**mk); gru.n_items = bench.WORKLOAD['n_items']
+gru = g4.GRU4Rec(**mk); gru.n_items = wl['n_items']
 for name, w in gru._init_host_weights().items():
     eng.set(name, w)
-items, offset, order, supports = bench.build_workload(3 * K)
+items, offset, order, supports = bench.build_workload(wl, 3 * K)
 P = supports.astype(np.float64) ** mk['sample_alpha']; P = P.cumsum() / P.sum(); P[-1] = 1
 eng.set_sampling_cdf(P.astype(np.float32)); eng.generate_samples()
 sched = _lib.Schedule(items, offset, order, mk['batch_size'], mk['n_sample'], mode=0)
